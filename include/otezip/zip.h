@@ -112,6 +112,19 @@ typedef struct zip_source otezip_src_buf;
 #define ZIP_ER_NOZIP 19
 #define ZIP_ER_INCONS 21
 #define ZIP_ER_RDONLY 25
+/* libzip's encryption error codes, for callers that use the names.  This subset has no per-archive error state: the
+ * calls fail with NULL / -1, and the reason an encrypted entry did not open is its status word
+ * (otezip_b200_entry_status: OTZ_ST_NOPASSWD, OTZ_ST_WRONGPASSWD, OTZ_ST_AUTH of include/otz_gpu.h). */
+#define ZIP_ER_ENCRNOTSUPP 24
+#define ZIP_ER_NOPASSWD 26
+#define ZIP_ER_WRONGPASSWD 27
+
+/* encryption methods (libzip values); only WinZip AES is implemented, traditional PKWARE encryption is not */
+#define ZIP_EM_NONE 0
+#define ZIP_EM_TRAD_PKWARE 1
+#define ZIP_EM_AES_128 0x0101
+#define ZIP_EM_AES_192 0x0102
+#define ZIP_EM_AES_256 0x0103
 
 #define ZIP_STAT_NAME 0x0001u
 #define ZIP_STAT_INDEX 0x0002u
@@ -164,6 +177,18 @@ int zip_replace(zip_t *za, zip_uint64_t index, zip_source_t *src);
 int zip_set_file_compression(zip_t *za, zip_uint64_t index, zip_int32_t comp, zip_uint32_t comp_flags);
 
 int otezip_method_from_string(const char *method_name);
+
+/* ---- WinZip AES encryption (method 99, AE-1 / AE-2; libzip's calls) ----
+ * Reading: an entry whose directory method is 99 is decrypted with the archive's default password (zip_fopen_index) or the
+ * one given (zip_fopen_index_encrypted), then decoded like any entry of its actual method; zip_stat keeps reporting 99.  A
+ * missing password, a wrong one and a failed authentication code make the open fail (otezip_b200_entry_status tells which:
+ * OTZ_ST_NOPASSWD, OTZ_ST_WRONGPASSWD, OTZ_ST_AUTH); no byte of an entry whose code does not match is ever handed out.
+ * Writing: zip_file_set_encryption on an entry added or replaced in this session makes zip_close write it as AE-2 (CRC field
+ * 0, the code is the integrity check) with a fresh random salt.  Passwords are wiped from the library's memory on zip_close. */
+int zip_set_default_password(zip_t *za, const char *password);   /* NULL clears it */
+zip_file_t *zip_fopen_index_encrypted(zip_t *za, zip_uint64_t index, zip_flags_t flags, const char *password);
+int zip_file_set_encryption(zip_t *za, zip_uint64_t index, zip_uint16_t method, const char *password);   /* NULL: the default */
+int zip_encryption_method_supported(zip_uint16_t method, int encode);
 
 /* ---- B200 build additions (not in the reference) ---- */
 /* Emit the device-side entry table of an archive opened for reading: n rows of struct otz_entry

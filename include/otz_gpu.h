@@ -56,6 +56,9 @@ extern "C" {
 #define OTZ_ST_TRUNCATED 8     /* input exhausted before the stream ended (Z_BUF_ERROR class) */
 #define OTZ_ST_OVERFLOW 9      /* stream produces more than uncomp_size bytes     dec:700-703, :791-793 */
 #define OTZ_ST_SIZE 10         /* method 93: total_out != uncomp_size             otezip.c:555 */
+#define OTZ_ST_NOPASSWD 11     /* WinZip AES entry (method 99) and no password given                 */
+#define OTZ_ST_WRONGPASSWD 12  /* password verification value does not match                         */
+#define OTZ_ST_AUTH 13         /* HMAC-SHA1 authentication code does not match: the ciphertext changed */
 #define OTZ_ST_PENDING 0x7F    /* never touched by a kernel (internal) */
 #define OTZ_ST_CODE(s) ((s) & 0xFF)
 #define OTZ_STF_CRC_MISMATCH 0x100 /* otezip.c:669: fatal only under otezip_verify_crc */
@@ -210,6 +213,36 @@ int otz_partition(const otz_entry *entries, uint32_t n, uint32_t parts, uint32_t
 int otz_extract_host_multi(otz_ctx *const *ctxs, uint32_t n_ctx, const uint8_t *archive, uint64_t archive_len,
 	const otz_entry *entries, uint32_t n, const otz_extract_opts *opts, uint8_t *out, uint64_t out_len, uint32_t *crc,
 	int32_t *status, uint32_t *produced);
+
+/* ---- WinZip AES (AE-1 / AE-2, method 99; k_aes.cuh) ----
+ * An encrypted payload is  salt (8/12/16 bytes for strength 1/2/3 = AES-128/192/256) | verification value (2) | ciphertext |
+ * authentication code (10).  Keys: PBKDF2-HMAC-SHA1(password, salt, 1000 iterations, 2*keylen + 2) = AES key | HMAC key |
+ * verification value.  Cipher: AES-CTR, little-endian counter from 1.  Code: HMAC-SHA1 over the ciphertext, first 10 bytes. */
+#define OTZ_AES_NOPASSWORD 0xFFFFu
+typedef struct otz_aes_entry {
+	uint64_t payload_ofs;   /* open: the payload in d_src;  seal: where the payload goes in d_out */
+	uint64_t data_ofs;      /* open: where the synthetic 30-byte local header goes in d_plain (the plaintext follows it);
+	                         * seal: the bytes to encrypt in d_in */
+	uint32_t size;          /* open: payload bytes (the directory's compressed size);  seal: bytes to encrypt */
+	uint16_t strength;      /* 1 / 2 / 3 */
+	uint16_t password;      /* index into passwords[]; OTZ_AES_NOPASSWORD = none (open reports OTZ_ST_NOPASSWD) */
+} otz_aes_entry;
+/* Decrypt n entries of d_src into the plaintext image d_plain (asynchronous): key derivation, then AES-CTR on the context's
+ * stream, the authentication codes on a side stream next to it.  Each entry of the image is a local header (signature, every
+ * other field zero) followed by the decrypted payload, so otz_plan_create / otz_extract_run decode the image as an archive.
+ * passwords[] are NUL-terminated byte strings.  d_src must stay valid until otz_aes_status. */
+int otz_aes_open(otz_ctx *ctx, const uint8_t *d_src, uint64_t src_len, const otz_aes_entry *ents, uint32_t n,
+	const char *const *passwords, uint32_t n_pw, uint8_t *d_plain, uint64_t plain_len);
+/* Join the side stream, clear the device key scratch and return the verdict of each entry of the last otz_aes_open
+ * (synchronises): OTZ_ST_OK, OTZ_ST_NOPASSWD, OTZ_ST_WRONGPASSWD or OTZ_ST_AUTH. */
+int otz_aes_status(otz_ctx *ctx, int32_t *status);
+/* Device time of the phases of the last otz_aes_open (valid after otz_aes_status), ms; any pointer may be NULL.  The
+ * authentication codes run beside the decryption: ms_mac counts from the end of the key derivation. */
+int otz_aes_times(otz_ctx *ctx, float *ms_kdf, float *ms_ctr, float *ms_mac);
+/* Encrypt n entries of d_in (e.g. otz_deflate_device_output) into d_out as salt | verification value | ciphertext | code,
+ * salts[16 * i ..] supplying the salt of entry i (its first 8/12/16 bytes).  Synchronises; the key scratch is cleared. */
+int otz_aes_seal(otz_ctx *ctx, const uint8_t *d_in, uint64_t in_len, const otz_aes_entry *ents, uint32_t n, const uint8_t *salts,
+	const char *const *passwords, uint32_t n_pw, uint8_t *d_out, uint64_t out_len);
 
 /* Policy helper shared by the host library and the tests: does a status word
  * mean "zip_fopen_index returns the buffer" under the given globals?

@@ -15,6 +15,7 @@
  */
 #include <errno.h>
 #include <fcntl.h>
+#include <sys/random.h>
 #include <sys/stat.h>
 #include <unistd.h>
 
@@ -33,6 +34,11 @@
  * u32 csize[n_chunks]}.  Each chunk is an independently decodable run of DEFLATE blocks (k_deflate.cuh). */
 #define OZ_EXTRA_ID 0x5A4Fu
 #define OZ_EXTRA_MAX_CHUNKS 16000u
+/* WinZip AES (AE-1 / AE-2): method 99, flag bit 0, extra field 0x9901 = {u16 vendor version 1|2, 'A' 'E', u8 strength 1-3,
+ * u16 actual method}; payload = salt (8/12/16) | verification value (2) | ciphertext | authentication code (10) */
+#define METHOD_AES 99u
+#define AES_EXTRA_ID 0x9901u
+#define AES_OVERHEAD(strength) (4u + 4u * (strength) + 2u + 10u)
 
 /* otezip.c:157-166 */
 int otezip_verify_crc = 0;
@@ -55,6 +61,7 @@ struct otz_window {               /* one decoded batch of consecutive entries */
 	uint32_t refs;                /* zip_file_t handles pointing into arena */
 	int current;
 	int orphan;                   /* its archive was closed while handles were still open: the last zip_fclose frees it */
+	uint32_t pw_gen;              /* default password its AES entries were decoded with (otz_archive.pw_gen) */
 };
 
 struct otz_pending {              /* a queued source (write path) */
@@ -63,6 +70,14 @@ struct otz_pending {              /* a queued source (write path) */
 	int owned;                    /* free(buf) after the archive is written */
 	int dirty;                    /* has bytes that zip_close must write (every new entry; a replaced existing one) */
 	int fast;                     /* zip_set_file_compression asked for level 1-3 (libzip: 1 = fastest) */
+	uint16_t enc;                 /* zip_file_set_encryption: AES strength 1-3, 0 = none */
+	char *pw;                     /* its password; NULL = the default password at zip_close */
+};
+
+struct otz_aesx {                 /* the 0x9901 field of an entry whose directory method is 99 */
+	uint16_t vendor;              /* 1 = AE-1, 2 = AE-2; 0 = no usable field (the entry is rejected with OTZ_ST_METHOD) */
+	uint8_t strength;
+	uint16_t method;              /* actual compression method */
 };
 
 static int index_enabled(void) {
@@ -85,6 +100,11 @@ struct otz_archive {
 	struct otz_pending *pend;     /* parallel to pub.entries for entries added in this session */
 	zip_uint64_t n_existing;      /* entries loaded from an existing archive (append mode) */
 	uint64_t append_ofs;          /* where new data starts in append mode */
+	/* encryption */
+	struct otz_aesx *aes;         /* per entry; vendor 0 for entries that are not AES-encrypted */
+	uint64_t aes_cap;
+	char *default_pw;
+	uint32_t pw_gen;              /* bumped by every zip_set_default_password */
 };
 #define OTZ_MAGIC 0x5a32424fu
 
@@ -158,6 +178,32 @@ static struct otz_archive *priv(zip_t *za) {
 
 static int is_valid(const zip_t *za) {
 	return za != NULL && za->fp != NULL; /* otezip.c:687-689 */
+}
+
+/* the AES field of entry i, or NULL when its directory method is not 99 (vendor 0: method 99 without a usable field) */
+static const struct otz_aesx *aes_of(const struct otz_archive *a, zip_uint64_t i) {
+	if (i >= a->pub.n_entries || a->pub.entries[i].method != METHOD_AES) {
+		return NULL;
+	}
+	static const struct otz_aesx none = { 0, 0, 0 };
+	return (a->aes && i < a->aes_cap) ? &a->aes[i] : &none;
+}
+
+/* compressed bytes the decoder sees: for an AES entry the ciphertext, without salt, verification value and code */
+static uint64_t inner_comp(const struct otz_archive *a, zip_uint64_t i) {
+	const struct otz_aesx *x = aes_of (a, i);
+	const uint64_t c = a->pub.entries[i].comp_size;
+	return (x && x->vendor && c >= AES_OVERHEAD (x->strength)) ? c - AES_OVERHEAD (x->strength) : c;
+}
+
+static void wipe_free(char *p) {
+	if (p) {
+		volatile char *v = p;
+		while (*v) {
+			*v++ = 0;
+		}
+		free (p);
+	}
 }
 
 #define OTZ_MAX_ENTRIES (1ull << 24)   /* ZIP64 lifts the 65,535 of the EOCD; this bounds the entry table */
@@ -310,7 +356,9 @@ static int load_central(struct otz_archive *a) {
 	za->entries = (struct otezip_entry *)calloc (n, sizeof (struct otezip_entry));
 	a->lfh64 = (uint64_t *)calloc (n, sizeof (uint64_t));
 	a->lfh64_cap = n;
-	if (!za->entries || !a->lfh64) {
+	a->aes = (struct otz_aesx *)calloc (n, sizeof (struct otz_aesx));
+	a->aes_cap = n;
+	if (!za->entries || !a->lfh64 || !a->aes) {
 		free (cd);
 		return ERR_READ;
 	}
@@ -337,17 +385,29 @@ static int load_central(struct otz_archive *a) {
 		e->external_attr = otezip_read_le32 (h + 38);
 		e->local_hdr_ofs = otezip_read_le32 (h + 42);
 		uint64_t comp64 = e->comp_size, uncomp64 = e->uncomp_size, lfh = e->local_hdr_ofs;
-		if (e->comp_size == 0xFFFFFFFFu || e->uncomp_size == 0xFFFFFFFFu || e->local_hdr_ofs == 0xFFFFFFFFu) {
-			/* ZIP64 extended information (APPNOTE 4.5.3): the escaped fields, in this order, 8 bytes each */
+		const int escaped = e->comp_size == 0xFFFFFFFFu || e->uncomp_size == 0xFFFFFFFFu || e->local_hdr_ofs == 0xFFFFFFFFu;
+		if (escaped || e->method == METHOD_AES) {
+			/* ZIP64 extended information (APPNOTE 4.5.3): the escaped fields, in this order, 8 bytes each;
+			 * WinZip AES field 0x9901 of a method-99 entry */
 			const uint8_t *x = h + 46 + fl;
 			size_t xo = 0;
-			int found = 0;
+			int found = !escaped;
 			while (xo + 4 <= xl) {
 				const size_t id = otezip_read_le16 (x + xo), sz = otezip_read_le16 (x + xo + 2);
 				if (xo + 4 + sz > xl) {
 					break;
 				}
-				if (id == 0x0001) {
+				if (id == AES_EXTRA_ID && e->method == METHOD_AES) {
+					const uint8_t *d = x + xo + 4;
+					const uint16_t ver = sz == 7 ? otezip_read_le16 (d) : 0, am = sz == 7 ? otezip_read_le16 (d + 5) : 0xFFFF;
+					if ((ver == 1 || ver == 2) && d[2] == 'A' && d[3] == 'E' && d[4] >= 1 && d[4] <= 3 &&
+						(am == OTEZIP_METHOD_STORE || am == OTEZIP_METHOD_DEFLATE || am == OTEZIP_METHOD_ZSTD)) {
+						a->aes[i].vendor = ver;
+						a->aes[i].strength = d[4];
+						a->aes[i].method = am;
+					}
+				}
+				if (id == 0x0001 && escaped) {
 					size_t q = xo + 4;
 					const size_t end = xo + 4 + sz;
 					found = 1;
@@ -371,7 +431,9 @@ static int load_central(struct otz_archive *a) {
 							lfh = (uint64_t)otezip_read_le32 (x + q) | ((uint64_t)otezip_read_le32 (x + q + 4) << 32);
 						}
 					}
-					break;
+					if (e->method != METHOD_AES) {
+						break;
+					}
 				}
 				xo += 4 + sz;
 			}
@@ -543,9 +605,12 @@ int zip_close(zip_t *za) {
 			if (a->pend[i].owned) {
 				free (a->pend[i].buf);
 			}
+			wipe_free (a->pend[i].pw);
 		}
 		free (a->pend);
 	}
+	wipe_free (a->default_pw);
+	free (a->aes);
 	free (za->entries);
 	free_windows (a);
 	if (a->image) {
@@ -660,13 +725,15 @@ static void drop_idle_windows(struct otz_archive *a) {
 	}
 }
 
-/* the zip-bomb rule of otezip.c:454-462, evaluated with the globals as they are NOW */
-static int bomb_rejects(const struct otezip_entry *e) {
-	if (otezip_ignore_zipbomb || e->comp_size == 0) {
+/* the zip-bomb rule of otezip.c:454-462, evaluated with the globals as they are NOW; an AES entry is judged by its
+ * ciphertext, what the decoder reads */
+static int bomb_rejects(const struct otz_archive *a, zip_uint64_t i) {
+	const uint64_t comp = inner_comp (a, i);
+	if (otezip_ignore_zipbomb || comp == 0) {
 		return 0;
 	}
-	uint64_t allowed = (uint64_t)e->comp_size * otezip_max_expansion_ratio + otezip_max_expansion_slack;
-	return (uint64_t)e->uncomp_size > allowed;
+	uint64_t allowed = comp * otezip_max_expansion_ratio + otezip_max_expansion_slack;
+	return (uint64_t)a->pub.entries[i].uncomp_size > allowed;
 }
 
 static int load_image(struct otz_archive *a) {
@@ -749,7 +816,9 @@ static uint32_t chunk_index_of(const struct otz_archive *a, const struct otezip_
  * otezip.c:403-487, in its order: LFH range and signature, payload range, zip-bomb rule, method, STORE size).  The
  * reference rejects such an entry BEFORE it allocates anything (otezip.c:454-462 precede the malloc at :470); here it
  * must not count towards the window's arena either: a crafted directory could otherwise claim gigabytes per entry. */
-static int32_t host_precheck(const struct otz_archive *a, const struct otezip_entry *e, uint64_t lfh) {
+static int32_t host_precheck(const struct otz_archive *a, zip_uint64_t i, const char *pw) {
+	const struct otezip_entry *e = &a->pub.entries[i];
+	const uint64_t lfh = entry_lfh (&a->pub, i);
 	const uint64_t len = a->image_len;
 	if (lfh > len || len - lfh < 30) {
 		return OTZ_ST_LFH_RANGE;
@@ -762,15 +831,28 @@ static int32_t host_precheck(const struct otz_archive *a, const struct otezip_en
 	if (data > len || (uint64_t)e->comp_size > MAX_PAYLOAD || (uint64_t)e->uncomp_size > MAX_PAYLOAD || data + e->comp_size > len) {
 		return OTZ_ST_DATA_RANGE;
 	}
-	if (bomb_rejects (e)) {
+	/* AES: the field must be usable and the payload hold salt, verification value and code; then the rules below apply
+	 * to the inner stream (ciphertext size, actual method) as they would to the same bytes stored unencrypted */
+	const struct otz_aesx *x = aes_of (a, i);
+	if (x && !x->vendor) {
+		return OTZ_ST_METHOD;
+	}
+	if (x && e->comp_size < AES_OVERHEAD (x->strength)) {
+		return OTZ_ST_DATA_RANGE;
+	}
+	if (bomb_rejects (a, i)) {
 		return OTZ_ST_ZIPBOMB;
 	}
-	if (e->method == OTEZIP_METHOD_STORE) {
-		if (e->comp_size != e->uncomp_size) {
+	const uint16_t method = x ? x->method : e->method;
+	if (method == OTEZIP_METHOD_STORE) {
+		if (inner_comp (a, i) != e->uncomp_size) {
 			return OTZ_ST_STORE_SIZE;
 		}
-	} else if (e->method != OTEZIP_METHOD_DEFLATE && e->method != OTEZIP_METHOD_ZSTD) {
+	} else if (method != OTEZIP_METHOD_DEFLATE && method != OTEZIP_METHOD_ZSTD) {
 		return OTZ_ST_METHOD;
+	}
+	if (x && !pw) {
+		return OTZ_ST_NOPASSWD;
 	}
 	return OTZ_ST_OK;
 }
@@ -783,18 +865,23 @@ static int32_t host_precheck(const struct otz_archive *a, const struct otezip_en
  * of the assembled entry does not match, the entry is decoded again as one plain stream.  (The CRC comparison is the
  * backstop, not a proof: with otezip_ref_compat = 1 and otezip_verify_crc = 0 a crafted index whose chunks decode
  * cleanly AND collide on CRC-32 could still differ from the sequential decode; OTEZIP_NO_INDEX=1 ignores the index.) */
-static struct otz_window *run_window(struct otz_archive *a, zip_uint64_t index) {
+/* AES entries (method 99) are not rows of that table: they form a second batch on the first device (aes_batch).
+ * pw_only != NULL: decode entry `index` alone with that password, into a window that is not cached (the caller owns it). */
+static int aes_batch(struct otz_archive *a, struct otz_window *w, const uint32_t *ks, uint32_t m, const char *pw, otz_ctx *ctx);
+
+static struct otz_window *run_window(struct otz_archive *a, zip_uint64_t index, const char *pw_only) {
 	zip_t *za = &a->pub;
 	otz_ctx **ctxs = NULL;
 	const uint32_t n_ctx = otezip_b200_ctxs (&ctxs);
 	if (!n_ctx || load_image (a) != 0) {
 		return NULL;
 	}
+	const char *pw = pw_only ? pw_only : a->default_pw;
 	const uint64_t budget = batch_budget ();
 	/* A request BELOW every decoded window (reverse iteration, zip_name_locate-driven access) would otherwise decode a full
 	 * window forward from each index it touches: start such a window up to half a budget earlier, so that the entries in
 	 * front of the requested one are decoded with it. */
-	int below_all = a->windows != NULL;
+	int below_all = a->windows != NULL && !pw_only;
 	zip_uint64_t lowest = za->n_entries;
 	for (struct otz_window *p = a->windows; p; p = p->next) {
 		below_all = below_all && index < p->first;
@@ -814,11 +901,11 @@ static struct otz_window *run_window(struct otz_archive *a, zip_uint64_t index) 
 	zip_uint64_t last = index;
 	uint64_t bytes = 0;
 	while (last < za->n_entries) {
-		if (below_all && last >= lowest) {
-			break;   /* (what follows is decoded already) */
+		if ((below_all && last >= lowest) || (pw_only && last > index)) {
+			break;   /* (what follows is decoded already; or the entry is decoded on its own) */
 		}
 		const struct otezip_entry *e = &za->entries[last];
-		uint64_t sz = host_precheck (a, e, entry_lfh (za, last)) == OTZ_ST_OK ? ((uint64_t)e->uncomp_size + 15) & ~15ULL : 0;
+		uint64_t sz = host_precheck (a, last, pw) == OTZ_ST_OK ? ((uint64_t)e->uncomp_size + 15) & ~15ULL : 0;
 		if (last > index && bytes + sz > budget) {
 			break;
 		}
@@ -829,16 +916,20 @@ static struct otz_window *run_window(struct otz_archive *a, zip_uint64_t index) 
 	/* rows of the device table: admitted entries first (compact), then their chunk rows */
 	int32_t *pre = (int32_t *)calloc (n ? n : 1, sizeof (int32_t));
 	uint32_t *rowof = (uint32_t *)calloc (n ? n : 1, sizeof (uint32_t));
-	if (!pre || !rowof) {
+	uint32_t *aes_ks = (uint32_t *)calloc (n ? n : 1, sizeof (uint32_t));
+	if (!pre || !rowof || !aes_ks) {
 		free (pre);
 		free (rowof);
+		free (aes_ks);
 		return NULL;
 	}
-	uint32_t n_adm = 0, n_rows = 0;
+	uint32_t n_adm = 0, n_rows = 0, n_aes = 0;
 	for (uint32_t k = 0; k < n; k++) {
-		pre[k] = host_precheck (a, &za->entries[index + k], entry_lfh (za, index + k));
+		pre[k] = host_precheck (a, index + k, pw);
 		rowof[k] = 0xFFFFFFFFu;
-		if (pre[k] == OTZ_ST_OK) {
+		if (pre[k] == OTZ_ST_OK && aes_of (a, index + k)) {
+			aes_ks[n_aes++] = k;
+		} else if (pre[k] == OTZ_ST_OK) {
 			uint32_t cb;
 			const uint8_t *cs;
 			uint64_t dofs;
@@ -865,16 +956,22 @@ static struct otz_window *run_window(struct otz_archive *a, zip_uint64_t index) 
 		free (row_crc);
 		free (pre);
 		free (rowof);
+		free (aes_ks);
 		return NULL;
 	}
 	w->first = index;
 	w->last = last;
+	w->pw_gen = a->pw_gen;
 	uint64_t out = 0;
 	uint32_t next_row = n_adm; /* chunk rows follow the entry rows */
 	for (uint32_t k = 0; k < n; k++) {
 		const struct otezip_entry *e = &za->entries[index + k];
 		w->ofs[k] = out;
 		if (pre[k] != OTZ_ST_OK) {
+			continue;
+		}
+		if (rowof[k] == 0xFFFFFFFFu) {   /* AES */
+			out += ((uint64_t)e->uncomp_size + 15) & ~15ULL;
 			continue;
 		}
 		otz_entry *t = &tab[rowof[k]];
@@ -955,26 +1052,35 @@ static struct otz_window *run_window(struct otz_archive *a, zip_uint64_t index) 
 		free (map);
 	}
 	for (uint32_t k = 0; k < n; k++) {
-		w->status[k] = pre[k] != OTZ_ST_OK ? pre[k] : row_status[rowof[k]];
-		w->crc[k] = pre[k] != OTZ_ST_OK ? 0u : row_crc[rowof[k]];
+		const int plain = pre[k] == OTZ_ST_OK && rowof[k] != 0xFFFFFFFFu;
+		w->status[k] = plain ? row_status[rowof[k]] : pre[k];
+		w->crc[k] = plain ? row_crc[rowof[k]] : 0u;
+	}
+	if (rc == OTZ_SUCCESS && n_aes) {
+		rc = aes_batch (a, w, aes_ks, n_aes, pw, ctxs[0]);
 	}
 	free (tab);
 	free (row_status);
 	free (row_crc);
 	free (pre);
 	free (rowof);
+	free (aes_ks);
 	if (rc != OTZ_SUCCESS) {
 		fprintf (stderr, "otezip-b200: GPU extract failed: %s\n", otz_last_error ());
 		free_window (w);
 		return NULL;
 	}
-	for (struct otz_window *p = a->windows; p; p = p->next) {
-		p->current = 0;
+	if (pw_only) {
+		w->orphan = 1;   /* not cached: freed by the last zip_fclose of its handles */
+	} else {
+		for (struct otz_window *p = a->windows; p; p = p->next) {
+			p->current = 0;
+		}
+		w->current = 1;
+		w->next = a->windows;
+		a->windows = w;
+		drop_idle_windows (a);
 	}
-	w->current = 1;
-	w->next = a->windows;
-	a->windows = w;
-	drop_idle_windows (a);
 	if (!a->last_status) {
 		a->last_status = (int32_t *)malloc (za->n_entries * sizeof (int32_t));
 		for (zip_uint64_t i = 0; a->last_status && i < za->n_entries; i++) {
@@ -987,6 +1093,137 @@ static struct otz_window *run_window(struct otz_archive *a, zip_uint64_t index) 
 	return w;
 }
 
+/* The AES entries ks[0..m) of window w (all past host_precheck): their payloads packed into one upload, each ciphertext
+ * 16-byte aligned; otz_aes_open decrypts them into a plaintext image of synthetic local headers; that image is decoded
+ * with the ordinary plan as an archive of plain entries (actual method, ciphertext size, directory CRC); the verdicts come
+ * last.  NOPASSWD / WRONGPASSWD / AUTH override the decode's status, and only entries that pass the authentication code
+ * are copied into the window's arena.  AE-2 stores no CRC (the code is the integrity check): its mismatch flag is dropped. */
+static int aes_batch(struct otz_archive *a, struct otz_window *w, const uint32_t *ks, uint32_t m, const char *pw, otz_ctx *ctx) {
+	zip_t *za = &a->pub;
+	otz_aes_entry *rows = (otz_aes_entry *)calloc (m, sizeof (otz_aes_entry));
+	otz_entry *tab = (otz_entry *)calloc (m, sizeof (otz_entry));
+	int32_t *st = (int32_t *)calloc (m, sizeof (int32_t)), *verdict = (int32_t *)calloc (m, sizeof (int32_t));
+	uint32_t *crc = (uint32_t *)calloc (m, sizeof (uint32_t));
+	uint8_t *h_src = NULL;
+	void *d_src = NULL, *d_plain = NULL, *d_out = NULL;
+	otz_plan *plan = NULL;
+	int rc = OTZ_ERR_NOMEM;
+	uint64_t src_len = 0, plain_len = 0, out_len = 0;
+	if (!rows || !tab || !st || !verdict || !crc) {
+		goto out;
+	}
+	for (uint32_t j = 0; j < m; j++) {
+		const zip_uint64_t i = w->first + ks[j];
+		const struct otezip_entry *e = &za->entries[i];
+		const struct otz_aesx *x = aes_of (a, i);
+		const uint64_t pre = 4u + 4u * x->strength + 2u;          /* salt + verification value */
+		rows[j].payload_ofs = ((src_len + pre + 15) & ~15ULL) - pre;
+		rows[j].size = e->comp_size;
+		rows[j].strength = x->strength;
+		rows[j].password = 0;
+		src_len = rows[j].payload_ofs + e->comp_size;
+		rows[j].data_ofs = ((plain_len + 30 + 15) & ~15ULL) - 30;
+		plain_len = rows[j].data_ofs + 30 + inner_comp (a, i);
+		tab[j].lfh_ofs = rows[j].data_ofs;
+		tab[j].out_ofs = out_len;
+		tab[j].comp_size = (uint32_t)inner_comp (a, i);
+		tab[j].uncomp_size = e->uncomp_size;
+		tab[j].crc32 = e->crc32;
+		tab[j].method = x->method;
+		tab[j].flags = 0;
+		out_len += ((uint64_t)e->uncomp_size + 15) & ~15ULL;
+	}
+	void *p = NULL;
+	if ((rc = otz_host_alloc (src_len + 64, &p)) != OTZ_SUCCESS) {
+		goto out;
+	}
+	h_src = (uint8_t *)p;
+	for (uint32_t j = 0; j < m; j++) {
+		const zip_uint64_t i = w->first + ks[j];
+		const uint8_t *h = a->image + entry_lfh (za, i);
+		const uint64_t data = entry_lfh (za, i) + 30u + otezip_read_le16 (h + 26) + otezip_read_le16 (h + 28);
+		memcpy (h_src + rows[j].payload_ofs, a->image + data, rows[j].size);
+	}
+	otz_extract_opts o;
+	o.ignore_zipbomb = otezip_ignore_zipbomb;
+	o.max_ratio = otezip_max_expansion_ratio;
+	o.max_slack = otezip_max_expansion_slack;
+	o.verify_only = 0;
+	if ((rc = otz_dev_alloc (ctx, src_len, &d_src)) != OTZ_SUCCESS || (rc = otz_dev_alloc (ctx, plain_len, &d_plain)) != OTZ_SUCCESS ||
+		(rc = otz_dev_alloc (ctx, out_len, &d_out)) != OTZ_SUCCESS || (rc = otz_h2d (ctx, d_src, h_src, src_len)) != OTZ_SUCCESS ||
+		(rc = otz_aes_open (ctx, (const uint8_t *)d_src, src_len, rows, m, &pw, 1, (uint8_t *)d_plain, plain_len)) != OTZ_SUCCESS) {
+		goto out;
+	}
+	rc = otz_plan_create (ctx, tab, m, &o, &plan);
+	if (rc == OTZ_SUCCESS) {
+		rc = otz_extract_run (ctx, plan, (const uint8_t *)d_plain, plain_len, (uint8_t *)d_out, out_len);
+	}
+	if (rc == OTZ_SUCCESS) {
+		rc = otz_extract_results (ctx, plan, crc, st);
+	}
+	{
+		const int src = otz_aes_status (ctx, verdict);   /* (always collected: it joins the side stream and clears the keys) */
+		rc = rc == OTZ_SUCCESS ? src : rc;
+	}
+	for (uint32_t j = 0; rc == OTZ_SUCCESS && j < m; j++) {
+		const zip_uint64_t i = w->first + ks[j];
+		int32_t s = st[j];
+		if (verdict[j] != OTZ_ST_OK) {
+			s = verdict[j];
+		} else if (aes_of (a, i)->vendor == 2) {
+			s &= ~OTZ_STF_CRC_MISMATCH;
+		}
+		w->status[ks[j]] = s;
+		w->crc[ks[j]] = verdict[j] == OTZ_ST_OK ? crc[j] : 0u;
+	}
+	/* one copy per run of authenticated entries that lie at the same distances in the device output and in the arena
+	 * (consecutive AES entries of the window, or separated only by rejected ones, whose slices are empty) */
+	for (uint32_t j = 0; rc == OTZ_SUCCESS && j < m;) {
+		if (verdict[j] != OTZ_ST_OK) {
+			j++;
+			continue;
+		}
+		uint32_t e = j + 1;
+		while (e < m && verdict[e] == OTZ_ST_OK && w->ofs[ks[e]] - w->ofs[ks[j]] == tab[e].out_ofs - tab[j].out_ofs) {
+			e++;
+		}
+		const uint64_t bytes = tab[e - 1].out_ofs + tab[e - 1].uncomp_size - tab[j].out_ofs;
+		if (bytes) {
+			rc = otz_d2h (ctx, w->arena + w->ofs[ks[j]], (const uint8_t *)d_out + tab[j].out_ofs, bytes);
+		}
+		j = e;
+	}
+	if (rc == OTZ_SUCCESS) {
+		rc = otz_sync (ctx);
+	}
+out:
+	if (plan) {
+		otz_plan_destroy (ctx, plan);
+	}
+	if (d_src) {
+		otz_dev_free (ctx, d_src);
+	}
+	if (d_plain) {
+		otz_dev_memset (ctx, d_plain, 0, plain_len);   /* (the plaintext does not outlive the batch on the device) */
+		otz_sync (ctx);
+		otz_dev_free (ctx, d_plain);
+	}
+	if (d_out) {
+		otz_dev_memset (ctx, d_out, 0, out_len);   /* (nor its decode, which includes entries that failed authentication) */
+		otz_sync (ctx);
+		otz_dev_free (ctx, d_out);
+	}
+	if (h_src) {
+		otz_host_free (h_src);
+	}
+	free (rows);
+	free (tab);
+	free (st);
+	free (verdict);
+	free (crc);
+	return rc;
+}
+
 int otezip_b200_entry_status(zip_t *za, zip_uint64_t index) {
 	struct otz_archive *a = priv (za);
 	if (!a || !a->last_status || index >= za->n_entries) {
@@ -995,40 +1232,13 @@ int otezip_b200_entry_status(zip_t *za, zip_uint64_t index) {
 	return a->last_status[index];
 }
 
-/* otezip.c:1315-1334 + :399-684 */
-zip_file_t *zip_fopen_index(zip_t *za, zip_uint64_t index, zip_flags_t flags) {
-	(void)flags;
-	struct otz_archive *a = priv (za);
-	if (!is_valid (za) || !a || index >= za->n_entries) {
-		return NULL;
-	}
-	if (za->mode == 1 && (index >= a->n_existing || (a->pend && a->pend[index].dirty))) {
-		return NULL; /* queued, not yet written */
-	}
-	struct otezip_entry *e = &za->entries[index];
-	struct otz_window *w = NULL;
-	for (struct otz_window *p = a->windows; p; p = p->next) {
-		if (index >= p->first && index < p->last) {
-			w = p;
-			break;
-		}
-	}
-	/* a batch decoded under other zip-bomb globals may have skipped this entry: decide again */
-	if (w) {
-		int st = w->status[index - w->first];
-		if (OTZ_ST_CODE (st) == OTZ_ST_ZIPBOMB && !bomb_rejects (e)) {
-			w = NULL;
-		}
-	}
-	if (!w) {
-		w = run_window (a, index);
-		if (!w) {
-			return NULL;
-		}
-	}
+/* The handle of entry `index` from window w, or NULL when the current globals reject its status. */
+static zip_file_t *hand_out(struct otz_archive *a, struct otz_window *w, zip_uint64_t index) {
+	struct otezip_entry *e = &a->pub.entries[index];
+	const struct otz_aesx *x = aes_of (a, index);
 	const uint32_t k = (uint32_t)(index - w->first);
 	int32_t st = w->status[k];
-	if (OTZ_ST_CODE (st) == OTZ_ST_OK && bomb_rejects (e)) {
+	if (OTZ_ST_CODE (st) == OTZ_ST_OK && bomb_rejects (a, index)) {
 		st = OTZ_ST_ZIPBOMB; /* the guard tightened since the batch ran */
 	}
 	if (OTZ_ST_CODE (st) == OTZ_ST_ZIPBOMB) { /* otezip.c:459, verbatim */
@@ -1036,7 +1246,8 @@ zip_file_t *zip_fopen_index(zip_t *za, zip_uint64_t index, zip_flags_t flags) {
 			e->name ? e->name : "<unknown>", e->uncomp_size);
 		return NULL;
 	}
-	if (OTZ_ST_CODE (st) != OTZ_ST_OK || (otezip_ref_compat && (st & OTZ_STF_REF_EOB) && !(e->method == OTEZIP_METHOD_ZSTD && zstd_frames ()))) {
+	const uint16_t method = x ? x->method : e->method;
+	if (OTZ_ST_CODE (st) != OTZ_ST_OK || (otezip_ref_compat && (st & OTZ_STF_REF_EOB) && !(method == OTEZIP_METHOD_ZSTD && zstd_frames ()))) {
 		return NULL;
 	}
 	if (st & OTZ_STF_CRC_MISMATCH) { /* otezip.c:669-678 */
@@ -1056,6 +1267,107 @@ zip_file_t *zip_fopen_index(zip_t *za, zip_uint64_t index, zip_flags_t flags) {
 	f->win = w;
 	w->refs++;
 	return &f->pub;
+}
+
+/* otezip.c:1315-1334 + :399-684 */
+zip_file_t *zip_fopen_index(zip_t *za, zip_uint64_t index, zip_flags_t flags) {
+	(void)flags;
+	struct otz_archive *a = priv (za);
+	if (!is_valid (za) || !a || index >= za->n_entries) {
+		return NULL;
+	}
+	if (za->mode == 1 && (index >= a->n_existing || (a->pend && a->pend[index].dirty))) {
+		return NULL; /* queued, not yet written */
+	}
+	struct otz_window *w = NULL;
+	for (struct otz_window *p = a->windows; p; p = p->next) {
+		if (index >= p->first && index < p->last) {
+			w = p;
+			break;
+		}
+	}
+	/* a batch decoded under other zip-bomb globals may have skipped this entry, and an AES entry decoded under another
+	 * default password must not be handed out: decide again */
+	if (w) {
+		int st = w->status[index - w->first];
+		if ((OTZ_ST_CODE (st) == OTZ_ST_ZIPBOMB && !bomb_rejects (a, index)) || (aes_of (a, index) && w->pw_gen != a->pw_gen)) {
+			w = NULL;
+		}
+	}
+	if (!w) {
+		w = run_window (a, index, NULL);
+		if (!w) {
+			return NULL;
+		}
+	}
+	return hand_out (a, w, index);
+}
+
+/* libzip: open an entry with this password instead of the default one.  The result is bound to the password: unless it is
+ * the default password (whose results are cached), the entry is decoded again, on its own. */
+zip_file_t *zip_fopen_index_encrypted(zip_t *za, zip_uint64_t index, zip_flags_t flags, const char *password) {
+	struct otz_archive *a = priv (za);
+	if (!is_valid (za) || !a || index >= za->n_entries) {
+		return NULL;
+	}
+	if (!password || !aes_of (a, index) || (a->default_pw && !strcmp (password, a->default_pw))) {
+		return zip_fopen_index (za, index, flags);
+	}
+	if (za->mode == 1 && (index >= a->n_existing || (a->pend && a->pend[index].dirty))) {
+		return NULL;
+	}
+	struct otz_window *w = run_window (a, index, password);
+	if (!w) {
+		return NULL;
+	}
+	zip_file_t *f = hand_out (a, w, index);
+	if (!f) {
+		free_window (w);
+	}
+	return f;
+}
+
+int zip_set_default_password(zip_t *za, const char *password) {
+	struct otz_archive *a = priv (za);
+	if (!is_valid (za) || !a) {
+		return -1;
+	}
+	char *copy = password ? strdup (password) : NULL;
+	if (password && !copy) {
+		return -1;
+	}
+	wipe_free (a->default_pw);
+	a->default_pw = copy;
+	a->pw_gen++;   /* cached AES results belong to the old password */
+	return 0;
+}
+
+int zip_encryption_method_supported(zip_uint16_t method, int encode) {
+	(void)encode;
+	return method == ZIP_EM_NONE || method == ZIP_EM_AES_128 || method == ZIP_EM_AES_192 || method == ZIP_EM_AES_256;
+}
+
+/* libzip: encrypt an entry added or replaced in this session (as zip_set_file_compression, entries already on disk are
+ * refused); ZIP_EM_NONE undoes it.  password NULL: the default password at zip_close. */
+int zip_file_set_encryption(zip_t *za, zip_uint64_t index, zip_uint16_t method, const char *password) {
+	struct otz_archive *a = priv (za);
+	if (!is_valid (za) || !a || index >= za->n_entries || za->mode != 1 || !a->pend || !zip_encryption_method_supported (method, 1)) {
+		return -1;
+	}
+	if (index < a->n_existing && !a->pend[index].dirty) {
+		return -1;
+	}
+	char *copy = password ? strdup (password) : NULL;
+	if (password && !copy) {
+		return -1;
+	}
+	wipe_free (a->pend[index].pw);
+	a->pend[index].pw = method == ZIP_EM_NONE ? NULL : copy;
+	if (method == ZIP_EM_NONE) {
+		wipe_free (copy);
+	}
+	a->pend[index].enc = method == ZIP_EM_NONE ? 0 : (uint16_t)(method & 0xFF);
+	return 0;
 }
 
 int zip_fclose(zip_file_t *zf) { /* otezip.c:1336-1343: the library owns zf->data */
@@ -1237,6 +1549,8 @@ int zip_file_replace(zip_t *za, zip_uint64_t index, zip_source_t *src, zip_flags
 	}
 	np.dirty = 1;
 	np.fast = a->pend[index].fast; /* the level asked for with zip_set_file_compression stays with the entry */
+	np.enc = a->pend[index].enc;   /* and so does the encryption asked for with zip_file_set_encryption */
+	np.pw = a->pend[index].pw;
 	if (a->pend[index].owned) {
 		free (a->pend[index].buf);
 	}
@@ -1268,14 +1582,14 @@ static int streaming_layout(void) {
 	return otezip_write_data_descriptors || (e && *e && *e != '0');
 }
 
-static int write_lfh(FILE *fp, const struct otezip_entry *e, const uint8_t *extra, uint16_t extra_len, int streaming) {
+static int write_lfh(FILE *fp, const struct otezip_entry *e, const uint8_t *extra, uint16_t extra_len, int streaming, int encrypted) {
 	uint8_t h[30];
 	uint16_t t, d;
 	size_t nl = strlen (e->name);
 	dos_now (&t, &d); /* the reference re-samples the clock here, otezip.c:1464-1467 */
 	otezip_write_le32 (h, SIG_LFH);
 	otezip_write_le16 (h + 4, 20);
-	otezip_write_le16 (h + 6, streaming ? 0x0008 : 0); /* bit 3: CRC and sizes follow the payload (APPNOTE 4.3.9) */
+	otezip_write_le16 (h + 6, (streaming ? 0x0008 : 0) | (encrypted ? 0x0001 : 0)); /* bit 3: CRC and sizes follow the payload (APPNOTE 4.3.9) */
 	otezip_write_le16 (h + 8, e->method);
 	otezip_write_le16 (h + 10, t);
 	otezip_write_le16 (h + 12, d);
@@ -1301,15 +1615,28 @@ static int write_descriptor(FILE *fp, const struct otezip_entry *e) {
 	return fwrite (h, 1, 16, fp) == 16 ? 0 : -1;
 }
 
-static uint32_t write_cdh(FILE *fp, const struct otezip_entry *e, uint64_t lfh_ofs, int streaming) {
-	uint8_t h[46], x[12];
+/* the 0x9901 field of an AES entry (11 bytes) */
+static void aes_extra(uint8_t *x, const struct otz_aesx *ax) {
+	otezip_write_le16 (x, AES_EXTRA_ID);
+	otezip_write_le16 (x + 2, 7);
+	otezip_write_le16 (x + 4, ax->vendor);
+	x[6] = 'A';
+	x[7] = 'E';
+	x[8] = ax->strength;
+	otezip_write_le16 (x + 9, ax->method);
+}
+
+static uint32_t write_cdh(FILE *fp, const struct otezip_entry *e, uint64_t lfh_ofs, int streaming, const struct otz_aesx *ax) {
+	uint8_t h[46], x[12 + 11];
 	size_t nl = strlen (e->name);
 	const int z64 = lfh_ofs >= 0xFFFFFFFFULL;
+	const int enc = ax && ax->vendor;
+	const uint16_t xl = (uint16_t)((z64 ? 12 : 0) + (enc ? 11 : 0));
 	memset (h, 0, sizeof (h));
 	otezip_write_le32 (h, SIG_CDH);
 	otezip_write_le16 (h + 4, 0x031e);
 	otezip_write_le16 (h + 6, z64 ? 45 : 20);
-	otezip_write_le16 (h + 8, streaming ? 0x0008 : 0);
+	otezip_write_le16 (h + 8, (streaming ? 0x0008 : 0) | (enc ? 0x0001 : 0));
 	otezip_write_le16 (h + 10, e->method);
 	otezip_write_le16 (h + 12, e->file_time);
 	otezip_write_le16 (h + 14, e->file_date);
@@ -1317,7 +1644,7 @@ static uint32_t write_cdh(FILE *fp, const struct otezip_entry *e, uint64_t lfh_o
 	otezip_write_le32 (h + 20, e->comp_size);
 	otezip_write_le32 (h + 24, e->uncomp_size);
 	otezip_write_le16 (h + 28, (uint16_t)nl);
-	otezip_write_le16 (h + 30, z64 ? 12 : 0);
+	otezip_write_le16 (h + 30, xl);
 	otezip_write_le32 (h + 38, e->external_attr);
 	otezip_write_le32 (h + 42, z64 ? 0xFFFFFFFFu : (uint32_t)lfh_ofs);
 	fwrite (h, 1, 46, fp);
@@ -1327,9 +1654,124 @@ static uint32_t write_cdh(FILE *fp, const struct otezip_entry *e, uint64_t lfh_o
 		otezip_write_le16 (x + 2, 8);
 		otezip_write_le32 (x + 4, (uint32_t)lfh_ofs);
 		otezip_write_le32 (x + 8, (uint32_t)(lfh_ofs >> 32));
-		fwrite (x, 1, 12, fp);
 	}
-	return (uint32_t)(46 + nl + (z64 ? 12 : 0));
+	if (enc) {
+		aes_extra (x + (z64 ? 12 : 0), ax);
+	}
+	if (xl) {
+		fwrite (x, 1, xl, fp);
+	}
+	return (uint32_t)(46 + nl + xl);
+}
+
+/* The encrypted entries of a write batch: sealed on the device straight from the compressor's dense arena (otz_aes_seal), then
+ * fetched.  *sealed[sofs[k] ..] holds salt | verification value | ciphertext | code of new entry k (sofs[k] = ~0 for entries
+ * that are not encrypted).  Salts come from getrandom(2), one per entry; without random bytes nothing is written. */
+#define SEAL_BATCH 65534u
+static int seal_entries(struct otz_archive *a, otz_ctx *ctx, otz_deflate_job *job, const zip_uint64_t *idx, zip_uint64_t n_new,
+	const uint64_t *out_ofs, const uint32_t *out_size, uint64_t out_total, uint8_t **sealed, uint64_t *sofs) {
+	zip_uint64_t m = 0;
+	uint64_t len = 0;
+	for (zip_uint64_t k = 0; k < n_new; k++) {
+		sofs[k] = ~0ULL;
+		const struct otz_pending *p = &a->pend[idx[k]];
+		if (p->enc) {
+			const uint64_t pre = 4u + 4u * p->enc + 2u;
+			sofs[k] = ((len + pre + 15) & ~15ULL) - pre;
+			len = sofs[k] + out_size[k] + AES_OVERHEAD (p->enc);
+			m++;
+		}
+	}
+	otz_aes_entry *rows = (otz_aes_entry *)calloc (m, sizeof (*rows));
+	const char **pws = (const char **)calloc (m, sizeof (*pws));
+	const char **uniq = (const char **)calloc (m < SEAL_BATCH ? m + 1 : SEAL_BATCH, sizeof (*uniq));
+	uint8_t *salts = (uint8_t *)calloc (m, 16);
+	void *d_out = NULL, *h = NULL;
+	int rc = -1;
+	if (!rows || !pws || !uniq || !salts) {
+		goto out;
+	}
+	uint32_t j = 0;
+	for (zip_uint64_t k = 0; k < n_new; k++) {
+		const struct otz_pending *p = &a->pend[idx[k]];
+		if (!p->enc) {
+			continue;
+		}
+		pws[j] = p->pw ? p->pw : a->default_pw;
+		if (!pws[j]) {
+			fprintf (stderr, "otezip-b200: no password for the encrypted entry '%s'\n", a->pub.entries[idx[k]].name);
+			goto out;
+		}
+		rows[j].payload_ofs = sofs[k];
+		rows[j].data_ofs = out_ofs[k];
+		rows[j].size = out_size[k];
+		rows[j].strength = p->enc;
+		j++;
+	}
+	for (uint64_t got = 0; got < 16 * m;) {
+		const ssize_t r = getrandom (salts + got, 16 * m - got, 0);
+		if (r <= 0 && errno != EINTR) {
+			fprintf (stderr, "otezip-b200: no random bytes for the salts: %s\n", strerror (errno));
+			goto out;
+		}
+		got += r > 0 ? (uint64_t)r : 0;
+	}
+	if (otz_host_alloc (len + 64, &h) != OTZ_SUCCESS || otz_dev_alloc (ctx, len, &d_out) != OTZ_SUCCESS) {
+		fprintf (stderr, "otezip-b200: %s\n", otz_last_error ());
+		goto out;
+	}
+	/* One otz_aes_seal per SEAL_BATCH entries (a call indexes at most 65,534 passwords).  Its password list holds each
+	 * distinct password once: an entry reuses the slot of the previous entry's password, or of any earlier one while the
+	 * list is short; otherwise (many per-entry passwords) it gets a slot of its own. */
+	for (zip_uint64_t b = 0; b < m; b += SEAL_BATCH) {
+		const uint32_t nb = (uint32_t)(m - b < SEAL_BATCH ? m - b : SEAL_BATCH);
+		uint32_t n_pw = 0;
+		for (uint32_t q = 0; q < nb; q++) {
+			const char *pw = pws[b + q];
+			uint32_t slot = n_pw;
+			if (n_pw && (uniq[n_pw - 1] == pw || !strcmp (uniq[n_pw - 1], pw))) {
+				slot = n_pw - 1;
+			} else if (n_pw <= 64) {
+				for (uint32_t u = 0; u < n_pw; u++) {
+					if (!strcmp (uniq[u], pw)) {
+						slot = u;
+						break;
+					}
+				}
+			}
+			if (slot == n_pw) {
+				uniq[n_pw++] = pw;
+			}
+			rows[b + q].password = (uint16_t)slot;
+		}
+		if (otz_aes_seal (ctx, otz_deflate_device_output (job), out_total, rows + b, nb, salts + 16 * b, uniq, n_pw, (uint8_t *)d_out, len) !=
+			OTZ_SUCCESS) {
+			fprintf (stderr, "otezip-b200: GPU encrypt failed: %s\n", otz_last_error ());
+			goto out;
+		}
+	}
+	if (otz_d2h (ctx, h, d_out, len) != OTZ_SUCCESS || otz_sync (ctx) != OTZ_SUCCESS) {
+		fprintf (stderr, "otezip-b200: GPU encrypt failed: %s\n", otz_last_error ());
+		goto out;
+	}
+	*sealed = (uint8_t *)h;
+	h = NULL;
+	rc = 0;
+out:
+	if (d_out) {
+		otz_dev_free (ctx, d_out);
+	}
+	if (h) {
+		otz_host_free (h);
+	}
+	if (salts) {
+		memset (salts, 0, 16 * m);
+	}
+	free (salts);
+	free (pws);
+	free (uniq);
+	free (rows);
+	return rc;
 }
 
 /* zip_close of a written archive: one GPU batch (CRC + DEFLATE/STORE decision), then LFH+payload per
@@ -1348,7 +1790,8 @@ static int finalize_archive(struct otz_archive *a) {
 			idx[n_new++] = i;
 		}
 	}
-	uint64_t *in_ofs = NULL, *out_ofs = NULL;
+	uint64_t *in_ofs = NULL, *out_ofs = NULL, *sofs = NULL;
+	uint8_t *sealed = NULL;
 	uint32_t *in_len = NULL, *out_size = NULL, *crc = NULL;
 	uint16_t *method = NULL, *method_out = NULL;
 	uint8_t *in = NULL, *out = NULL;
@@ -1357,6 +1800,16 @@ static int finalize_archive(struct otz_archive *a) {
 	if (fseek (za->fp, (long)pos, SEEK_SET) != 0) {
 		free (idx);
 		return -1;
+	}
+	if (za->n_entries > a->aes_cap) {
+		struct otz_aesx *na = (struct otz_aesx *)realloc (a->aes, za->n_entries * sizeof (*na));
+		if (!na) {
+			free (idx);
+			return -1;
+		}
+		memset (na + a->aes_cap, 0, (za->n_entries - a->aes_cap) * sizeof (*na));
+		a->aes = na;
+		a->aes_cap = za->n_entries;
 	}
 	if (za->n_entries > a->lfh64_cap) {
 		uint64_t *nl64 = (uint64_t *)realloc (a->lfh64, za->n_entries * sizeof (uint64_t));
@@ -1380,7 +1833,8 @@ static int finalize_archive(struct otz_archive *a) {
 		crc = (uint32_t *)calloc (n_new, 4);
 		method = (uint16_t *)calloc (n_new, 2);
 		method_out = (uint16_t *)calloc (n_new, 2);
-		if (!in_ofs || !out_ofs || !in_len || !out_size || !crc || !method || !method_out) {
+		sofs = (uint64_t *)calloc (n_new, 8);
+		if (!in_ofs || !out_ofs || !in_len || !out_size || !crc || !method || !method_out || !sofs) {
 			goto done;
 		}
 		uint64_t total = 0;
@@ -1428,6 +1882,13 @@ static int finalize_archive(struct otz_archive *a) {
 				ok = 0;
 			}
 		}
+		int any_enc = 0;
+		for (zip_uint64_t k = 0; k < n_new; k++) {
+			any_enc |= a->pend[idx[k]].enc != 0;
+		}
+		if (ok && any_enc && seal_entries (a, ctx, job, idx, n_new, out_ofs, out_size, out_total, &sealed, sofs) != 0) {
+			ok = 0;
+		}
 		if (d_in) {
 			otz_dev_free (ctx, d_in);
 		}
@@ -1441,15 +1902,27 @@ static int finalize_archive(struct otz_archive *a) {
 		}
 		for (zip_uint64_t k = 0; k < n_new; k++) {
 			struct otezip_entry *e = &za->entries[idx[k]];
-			e->crc32 = crc[k];
-			e->comp_size = out_size[k];
-			e->method = method_out[k];
+			const uint16_t enc = a->pend[idx[k]].enc;
+			e->crc32 = enc ? 0u : crc[k];   /* AE-2: no CRC of the plaintext in the clear */
+			e->comp_size = out_size[k] + (enc ? AES_OVERHEAD (enc) : 0u);
+			e->method = enc ? (uint16_t)METHOD_AES : method_out[k];
+			a->aes[idx[k]].vendor = enc ? 2 : 0;
+			a->aes[idx[k]].strength = (uint8_t)enc;
+			a->aes[idx[k]].method = method_out[k];
 			e->local_hdr_ofs = (uint32_t)pos;   /* (the reference gives up beyond 4 GiB, otezip.c:1140; ZIP64 here) */
 			a->lfh64[idx[k]] = pos;
 			/* chunk index for multi-chunk DEFLATE entries */
 			uint8_t *extra = NULL;
 			uint16_t extra_len = 0;
-			if (index_enabled () && e->method == OTEZIP_METHOD_DEFLATE && n_chunks[k] >= 2 && n_chunks[k] <= OZ_EXTRA_MAX_CHUNKS) {
+			if (enc) {
+				extra_len = 11;
+				extra = (uint8_t *)malloc (extra_len);
+				if (!extra) {
+					ok = 0;
+					break;
+				}
+				aes_extra (extra, &a->aes[idx[k]]);
+			} else if (index_enabled () && e->method == OTEZIP_METHOD_DEFLATE && n_chunks[k] >= 2 && n_chunks[k] <= OZ_EXTRA_MAX_CHUNKS) {
 				extra_len = (uint16_t)(4 + 12 + 4 * n_chunks[k]);
 				extra = (uint8_t *)calloc (1, extra_len);
 				if (extra) {
@@ -1465,14 +1938,15 @@ static int finalize_archive(struct otz_archive *a) {
 					extra_len = 0;
 				}
 			}
-			int wrc = write_lfh (za->fp, e, extra, extra_len, streaming);
+			int wrc = write_lfh (za->fp, e, extra, extra_len, streaming, enc != 0);
 			free (extra);
-			if (wrc != 0 || (out_size[k] && fwrite (out + out_ofs[k], 1, out_size[k], za->fp) != out_size[k]) ||
+			const uint8_t *payload = enc ? sealed + sofs[k] : out + out_ofs[k];
+			if (wrc != 0 || (e->comp_size && fwrite (payload, 1, e->comp_size, za->fp) != e->comp_size) ||
 				(streaming && write_descriptor (za->fp, e) != 0)) {
 				ok = 0;
 				break;
 			}
-			pos += 30 + strlen (e->name) + extra_len + out_size[k] + (streaming ? 16u : 0u);
+			pos += 30 + strlen (e->name) + extra_len + e->comp_size + (streaming ? 16u : 0u);
 		}
 		free (first_chunk);
 		free (n_chunks);
@@ -1484,7 +1958,8 @@ static int finalize_archive(struct otz_archive *a) {
 	{
 		uint64_t cd_size = 0;
 		for (zip_uint64_t i = 0; i < za->n_entries; i++) {
-			cd_size += write_cdh (za->fp, &za->entries[i], entry_lfh (za, i), streaming && (!a->n_existing || i >= a->n_existing || (a->pend && a->pend[i].dirty)));
+			cd_size += write_cdh (za->fp, &za->entries[i], entry_lfh (za, i), streaming && (!a->n_existing || i >= a->n_existing || (a->pend && a->pend[i].dirty)),
+				aes_of (a, i));
 		}
 		/* otezip.c:1561-1590 truncates the counts to 16 bits and fails beyond 4 GiB (:1264); here the ZIP64 record and
 		 * locator (APPNOTE 4.3.14-4.3.15) are written whenever a field does not fit */
@@ -1547,5 +2022,9 @@ done:
 	free (crc);
 	free (method);
 	free (method_out);
+	free (sofs);
+	if (sealed) {
+		otz_host_free (sealed);
+	}
 	return rc;
 }

@@ -44,6 +44,11 @@ __device__ unsigned long long g_otz_violations[OTZ_CHK_SLOTS];
 #define OTZ_CK_ZS_REC 14        // k_zstd_seq: sequence record stored below the literals of the entry's token scratch
 #define OTZ_CK_ZS_LIT 15        // k_zstd_lit: literals of a block outside the entry's token scratch
 #define OTZ_CK_DFL_PAIR 16      // k_deflate_chunks: (token, way) pair of the second search pass outside the window / the chunk
+#define OTZ_CK_AES_RK 17        // k_aes_kdf / k_aes_ctr: round-key word beyond the 60 of AES-256
+#define OTZ_CK_AES_TAB 18       // k_aes_ctr: T-table / S-box slot beyond 256
+#define OTZ_CK_AES_WORK 19      // k_aes_ctr / k_aes_mac: work-list or job index out of range
+#define OTZ_CK_AES_OUT 20       // k_aes_ctr: plaintext-image / ciphertext store outside the output buffer
+#define OTZ_CK_AES_IN 21        // k_aes_ctr: load outside the input buffer
 
 #define OTZ_SIG_LFH 0x04034b50u
 #define OTZ_MAX_PAYLOAD (2ull * 1024ull * 1024ull * 1024ull)  // otezip.c:102

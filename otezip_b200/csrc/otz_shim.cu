@@ -17,6 +17,7 @@
 #include "k_deflate.cuh"
 #include "k_resolve.cuh"
 #include "k_zstd_tok.cuh"
+#include "k_aes.cuh"
 #include "otz_common.cuh"
 
 static thread_local char g_err[512] = "";
@@ -75,6 +76,7 @@ struct otz_ctx {
 	void *h_res;            // pinned staging of its per-entry results
 	uint64_t h_res_bytes;
 	uint64_t sym_limit;     // OTZ_SEG_SYM_LIMIT: cap of the symbol buffer in elements (tests: streams that do not fit are walked by one warp)
+	struct OtzAesRun *aes;  // device state of the last otz_aes_open / otz_aes_seal (created on first use)
 };
 
 struct otz_plan {
@@ -256,6 +258,7 @@ extern "C" int otz_ctx_create(int device, otz_ctx **out) {
 	return OTZ_SUCCESS;
 }
 
+static void aes_destroy(otz_ctx *c);
 extern "C" void otz_ctx_destroy(otz_ctx *c) {
 	if (!c) {
 		return;
@@ -270,6 +273,7 @@ extern "C" void otz_ctx_destroy(otz_ctx *c) {
 	cudaFree(c->d_sym_cache);
 	cudaFree(c->d_ztok_cache);
 	cudaFree(c->d_spec_tmp);
+	aes_destroy(c);
 	for (size_t k = 0; k < c->pc_plans.size(); k++) {
 		otz_plan_destroy(c->pipe[k & 1], c->pc_plans[k]);
 	}
@@ -1927,4 +1931,305 @@ extern "C" int otz_deflate_host(otz_ctx *c, const uint8_t *in, uint64_t in_bytes
 	}
 	otz_deflate_destroy(c, j);
 	return rc;
+}
+
+// ---------------------------------------------------------------- WinZip AES (k_aes.cuh)
+struct OtzAesRun {
+	cudaStream_t side;        // the authentication codes run here, beside CTR and the decode
+	cudaEvent_t ev[4];        // KDF start, KDF end, CTR end, MAC end
+	OtzAesJob *d_jobs;
+	OtzAesWork *d_work;
+	uint32_t *d_order;
+	OtzAesKeys *d_keys;
+	int32_t *d_verdict, *d_auth;
+	uint8_t *d_pw, *d_salts;
+	uint32_t *d_pw_ofs;
+	uint64_t pw_bytes;
+	uint32_t n;
+	bool open_pending;
+};
+
+static void aes_free_run(OtzAesRun *r) {
+	cudaFree(r->d_jobs);
+	cudaFree(r->d_work);
+	cudaFree(r->d_order);
+	cudaFree(r->d_keys);
+	cudaFree(r->d_verdict);
+	cudaFree(r->d_auth);
+	cudaFree(r->d_pw);
+	cudaFree(r->d_salts);
+	cudaFree(r->d_pw_ofs);
+	r->d_jobs = nullptr;
+	r->d_work = nullptr;
+	r->d_order = nullptr;
+	r->d_keys = nullptr;
+	r->d_verdict = r->d_auth = nullptr;
+	r->d_pw = r->d_salts = nullptr;
+	r->d_pw_ofs = nullptr;
+}
+
+static int aes_wipe(otz_ctx *c, OtzAesRun *r);
+static void aes_destroy(otz_ctx *c) {
+	OtzAesRun *r = c->aes;
+	if (!r) {
+		return;
+	}
+	cudaStreamSynchronize(r->side);
+	aes_wipe(c, r);
+	cudaStreamSynchronize(c->stream);
+	aes_free_run(r);
+	for (auto &e : r->ev) {
+		cudaEventDestroy(e);
+	}
+	cudaStreamDestroy(r->side);
+	delete r;
+	c->aes = nullptr;
+}
+
+static int aes_run(otz_ctx *c, OtzAesRun **out) {
+	if (!c->aes) {
+		OtzAesRun *r = new (std::nothrow) OtzAesRun();
+		if (!r) {
+			return OTZ_ERR_NOMEM;
+		}
+		c->aes = r;
+		CK(cudaStreamCreateWithFlags(&r->side, cudaStreamNonBlocking));
+		for (auto &e : r->ev) {
+			CK(cudaEventCreate(&e));
+		}
+	}
+	*out = c->aes;
+	return OTZ_SUCCESS;
+}
+
+static uint32_t aes_salt_bytes(uint16_t strength) { return 4u + 4u * strength; }
+
+// Clear the secrets of a run on the device (round keys, HMAC states, passwords), ordered after its kernels on the stream.
+static int aes_wipe(otz_ctx *c, OtzAesRun *r) {
+	if (r->n && r->d_keys) {
+		CK(cudaMemsetAsync(r->d_keys, 0, sizeof(OtzAesKeys) * r->n, c->stream));
+	}
+	if (r->pw_bytes && r->d_pw) {
+		CK(cudaMemsetAsync(r->d_pw, 0, r->pw_bytes, c->stream));
+	}
+	return OTZ_SUCCESS;
+}
+
+// Upload the jobs, the CTR work list, the longest-first order and the passwords; allocate keys and verdicts.
+static int aes_stage(otz_ctx *c, OtzAesRun *r, const std::vector<OtzAesJob> &jobs, const char *const *passwords, uint32_t n_pw) {
+	const uint32_t n = (uint32_t)jobs.size();
+	std::vector<OtzAesWork> work;
+	for (uint32_t i = 0; i < n; i++) {
+		const uint32_t nc = std::max<uint32_t>(1, (uint32_t)(((uint64_t)jobs[i].len + OTZ_AES_CHUNK - 1) / OTZ_AES_CHUNK));
+		for (uint32_t k = 0; k < nc; k++) {
+			work.push_back({ i, k });
+		}
+	}
+	std::vector<uint32_t> order(n);
+	for (uint32_t i = 0; i < n; i++) {
+		order[i] = i;
+	}
+	std::stable_sort(order.begin(), order.end(), [&](uint32_t a, uint32_t b) { return jobs[a].len > jobs[b].len; });
+	std::vector<uint32_t> pw_ofs(n_pw + 1, 0);
+	std::vector<uint8_t> pw;
+	for (uint32_t k = 0; k < n_pw; k++) {
+		const char *p = passwords[k] ? passwords[k] : "";
+		pw.insert(pw.end(), p, p + strlen(p));
+		pw_ofs[k + 1] = (uint32_t)pw.size();
+	}
+	r->n = n;
+	r->pw_bytes = pw.size();
+	int rc;
+	if ((rc = upload(&r->d_jobs, jobs, c->stream)) != OTZ_SUCCESS || (rc = upload(&r->d_work, work, c->stream)) != OTZ_SUCCESS ||
+		(rc = upload(&r->d_order, order, c->stream)) != OTZ_SUCCESS || (rc = upload(&r->d_pw, pw, c->stream)) != OTZ_SUCCESS ||
+		(rc = upload(&r->d_pw_ofs, pw_ofs, c->stream)) != OTZ_SUCCESS) {
+		return rc;
+	}
+	std::fill(pw.begin(), pw.end(), 0);   // (the host copy of the passwords)
+	CK(cudaMalloc(&r->d_keys, sizeof(OtzAesKeys) * std::max<uint32_t>(n, 1)));
+	CK(cudaMalloc(&r->d_verdict, sizeof(int32_t) * std::max<uint32_t>(n, 1)));
+	CK(cudaMalloc(&r->d_auth, sizeof(int32_t) * std::max<uint32_t>(n, 1)));
+	CK(cudaMemsetAsync(r->d_auth, 0, sizeof(int32_t) * std::max<uint32_t>(n, 1), c->stream));
+	return OTZ_SUCCESS;
+}
+
+extern "C" int otz_aes_open(otz_ctx *c, const uint8_t *d_src, uint64_t src_len, const otz_aes_entry *ents, uint32_t n,
+	const char *const *passwords, uint32_t n_pw, uint8_t *d_plain, uint64_t plain_len) {
+	if (!c || (n && (!ents || !d_src || !d_plain)) || (n_pw && !passwords) || n_pw >= OTZ_AES_NOPASSWORD) {
+		snprintf(g_err, sizeof(g_err), "otz_aes_open: missing buffer or more than %u passwords", OTZ_AES_NOPASSWORD - 1);
+		return OTZ_ERR_ARG;
+	}
+	CK(cudaSetDevice(c->device));
+	OtzAesRun *r;
+	int rc = aes_run(c, &r);
+	if (rc != OTZ_SUCCESS) {
+		return rc;
+	}
+	if (r->open_pending) {
+		snprintf(g_err, sizeof(g_err), "otz_aes_open: the previous run was not collected with otz_aes_status");
+		return OTZ_ERR_ARG;
+	}
+	CK(cudaStreamSynchronize(r->side));
+	aes_free_run(r);
+	std::vector<OtzAesJob> jobs(n);
+	for (uint32_t i = 0; i < n; i++) {
+		const otz_aes_entry &e = ents[i];
+		const uint32_t sl = aes_salt_bytes(e.strength);
+		if (e.strength < 1 || e.strength > 3 || e.size < sl + 2 + 10 || e.payload_ofs > src_len || src_len - e.payload_ofs < e.size ||
+			e.data_ofs > plain_len || plain_len - e.data_ofs < 30ull + e.size - sl - 12) {
+			snprintf(g_err, sizeof(g_err), "otz_aes_open: entry %u outside its buffers or of unknown strength", i);
+			return OTZ_ERR_ARG;
+		}
+		OtzAesJob &j = jobs[i];
+		j.salt = e.payload_ofs;
+		j.pwv = e.payload_ofs + sl;
+		j.src = e.payload_ofs + sl + 2;
+		j.len = e.size - sl - 12;
+		j.mac = j.src + j.len;
+		j.hdr = e.data_ofs;
+		j.dst = e.data_ofs + 30;
+		j.strength = e.strength;
+		j.pw = e.password < n_pw ? e.password : (uint16_t)OTZ_AES_NOPW;
+	}
+	if ((rc = aes_stage(c, r, jobs, passwords, n_pw)) != OTZ_SUCCESS) {
+		return rc;
+	}
+	CK(cudaEventRecord(r->ev[0], c->stream));
+	if (n) {
+		k_aes_kdf<<<(4 * n + OTZ_AES_KDF_THREADS - 1) / OTZ_AES_KDF_THREADS, OTZ_AES_KDF_THREADS, 0, c->stream>>>(r->d_jobs, n, r->d_pw,
+			r->d_pw_ofs, n_pw, d_src, const_cast<uint8_t *>(d_src), src_len, 0, r->d_keys, r->d_verdict);
+		CK(cudaGetLastError());
+		c->launches++;
+	}
+	CK(cudaEventRecord(r->ev[1], c->stream));
+	CK(cudaStreamWaitEvent(r->side, r->ev[1], 0));
+	if (n) {
+		uint32_t nw = 0;
+		for (const OtzAesJob &j : jobs) {
+			nw += std::max<uint32_t>(1, (uint32_t)(((uint64_t)j.len + OTZ_AES_CHUNK - 1) / OTZ_AES_CHUNK));
+		}
+		k_aes_ctr<<<nw, OTZ_AES_CTR_THREADS, 0, c->stream>>>(r->d_jobs, n, r->d_work, nw, r->d_keys, r->d_verdict, d_src, src_len,
+			d_plain, plain_len, 1);
+		CK(cudaGetLastError());
+		k_aes_mac<<<(n + 127) / 128, 128, 0, r->side>>>(r->d_jobs, r->d_order, n, r->d_keys, r->d_verdict, d_src,
+			const_cast<uint8_t *>(d_src), src_len, 0, r->d_auth);
+		CK(cudaGetLastError());
+		c->launches += 2;
+	}
+	CK(cudaEventRecord(r->ev[2], c->stream));
+	CK(cudaEventRecord(r->ev[3], r->side));
+	r->open_pending = true;
+	return OTZ_SUCCESS;
+}
+
+extern "C" int otz_aes_status(otz_ctx *c, int32_t *status) {
+	if (!c || !c->aes || !c->aes->open_pending) {
+		return OTZ_ERR_ARG;
+	}
+	CK(cudaSetDevice(c->device));
+	OtzAesRun *r = c->aes;
+	r->open_pending = false;
+	CK(cudaStreamWaitEvent(c->stream, r->ev[3], 0));
+	const uint32_t n = r->n;
+	std::vector<int32_t> v(std::max<uint32_t>(n, 1)), a(std::max<uint32_t>(n, 1));
+	int rc = aes_wipe(c, r);
+	if (rc != OTZ_SUCCESS) {
+		return rc;
+	}
+	if (n) {
+		CK(cudaMemcpyAsync(v.data(), r->d_verdict, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, c->stream));
+		CK(cudaMemcpyAsync(a.data(), r->d_auth, sizeof(int32_t) * n, cudaMemcpyDeviceToHost, c->stream));
+	}
+	CK(cudaStreamSynchronize(c->stream));
+	for (uint32_t i = 0; status && i < n; i++) {
+		status[i] = v[i] != OTZ_ST_OK ? v[i] : a[i] ? OTZ_ST_AUTH : OTZ_ST_OK;
+	}
+	return OTZ_SUCCESS;
+}
+
+extern "C" int otz_aes_times(otz_ctx *c, float *ms_kdf, float *ms_ctr, float *ms_mac) {
+	if (!c || !c->aes) {
+		return OTZ_ERR_ARG;
+	}
+	CK(cudaSetDevice(c->device));
+	OtzAesRun *r = c->aes;
+	CK(cudaEventSynchronize(r->ev[3]));
+	CK(cudaEventSynchronize(r->ev[2]));
+	if (ms_kdf) {
+		CK(cudaEventElapsedTime(ms_kdf, r->ev[0], r->ev[1]));
+	}
+	if (ms_ctr) {
+		CK(cudaEventElapsedTime(ms_ctr, r->ev[1], r->ev[2]));
+	}
+	if (ms_mac) {
+		CK(cudaEventElapsedTime(ms_mac, r->ev[1], r->ev[3]));
+	}
+	return OTZ_SUCCESS;
+}
+
+extern "C" int otz_aes_seal(otz_ctx *c, const uint8_t *d_in, uint64_t in_len, const otz_aes_entry *ents, uint32_t n, const uint8_t *salts,
+	const char *const *passwords, uint32_t n_pw, uint8_t *d_out, uint64_t out_len) {
+	if (!c || (n && (!ents || !salts || !d_out)) || (n_pw && !passwords) || n_pw >= OTZ_AES_NOPASSWORD) {
+		snprintf(g_err, sizeof(g_err), "otz_aes_seal: missing buffer or more than %u passwords", OTZ_AES_NOPASSWORD - 1);
+		return OTZ_ERR_ARG;
+	}
+	CK(cudaSetDevice(c->device));
+	OtzAesRun *r;
+	int rc = aes_run(c, &r);
+	if (rc != OTZ_SUCCESS) {
+		return rc;
+	}
+	if (r->open_pending) {
+		snprintf(g_err, sizeof(g_err), "otz_aes_seal: the previous otz_aes_open was not collected with otz_aes_status");
+		return OTZ_ERR_ARG;
+	}
+	CK(cudaStreamSynchronize(r->side));
+	aes_free_run(r);
+	std::vector<OtzAesJob> jobs(n);
+	for (uint32_t i = 0; i < n; i++) {
+		const otz_aes_entry &e = ents[i];
+		const uint32_t sl = aes_salt_bytes(e.strength);
+		if (e.strength < 1 || e.strength > 3 || e.password >= n_pw || (e.size && !d_in) || e.data_ofs > in_len || in_len - e.data_ofs < e.size ||
+			e.payload_ofs > out_len || out_len - e.payload_ofs < (uint64_t)e.size + sl + 12) {
+			snprintf(g_err, sizeof(g_err), "otz_aes_seal: entry %u outside its buffers, of unknown strength or without a password", i);
+			return OTZ_ERR_ARG;
+		}
+		OtzAesJob &j = jobs[i];
+		j.salt = 16ull * i;
+		j.hdr = e.payload_ofs;
+		j.pwv = e.payload_ofs + sl;
+		j.dst = e.payload_ofs + sl + 2;
+		j.src = e.data_ofs;
+		j.len = e.size;
+		j.mac = j.dst + j.len;
+		j.strength = e.strength;
+		j.pw = e.password;
+	}
+	if ((rc = aes_stage(c, r, jobs, passwords, n_pw)) != OTZ_SUCCESS) {
+		return rc;
+	}
+	if (n) {
+		std::vector<uint8_t> sv(salts, salts + 16ull * n);
+		if ((rc = upload(&r->d_salts, sv, c->stream)) != OTZ_SUCCESS) {
+			return rc;
+		}
+		uint32_t nw = 0;
+		for (const OtzAesJob &j : jobs) {
+			nw += std::max<uint32_t>(1, (uint32_t)(((uint64_t)j.len + OTZ_AES_CHUNK - 1) / OTZ_AES_CHUNK));
+		}
+		k_aes_kdf<<<(4 * n + OTZ_AES_KDF_THREADS - 1) / OTZ_AES_KDF_THREADS, OTZ_AES_KDF_THREADS, 0, c->stream>>>(r->d_jobs, n, r->d_pw,
+			r->d_pw_ofs, n_pw, r->d_salts, d_out, out_len, 1, r->d_keys, r->d_verdict);
+		CK(cudaGetLastError());
+		k_aes_ctr<<<nw, OTZ_AES_CTR_THREADS, 0, c->stream>>>(r->d_jobs, n, r->d_work, nw, r->d_keys, r->d_verdict, d_in, in_len, d_out,
+			out_len, 0);
+		CK(cudaGetLastError());
+		k_aes_mac<<<(n + 127) / 128, 128, 0, c->stream>>>(r->d_jobs, r->d_order, n, r->d_keys, r->d_verdict, d_out, d_out, out_len, 1, r->d_auth);
+		CK(cudaGetLastError());
+		c->launches += 3;
+	}
+	if ((rc = aes_wipe(c, r)) != OTZ_SUCCESS) {
+		return rc;
+	}
+	CK(cudaStreamSynchronize(c->stream));
+	return OTZ_SUCCESS;
 }

@@ -39,6 +39,16 @@ ST_OK = 0
 STF_CRC_MISMATCH, STF_REF_EOB, STF_SHORT = 0x100, 0x200, 0x400
 
 
+class OtzAesEntry(C.Structure):  # struct otz_aes_entry
+    _fields_ = [("payload_ofs", C.c_uint64), ("data_ofs", C.c_uint64), ("size", C.c_uint32), ("strength", C.c_uint16),
+                ("password", C.c_uint16)]
+
+
+AES_ENTRY_DTYPE = np.dtype([("payload_ofs", "<u8"), ("data_ofs", "<u8"), ("size", "<u4"), ("strength", "<u2"), ("password", "<u2")])
+assert AES_ENTRY_DTYPE.itemsize == C.sizeof(OtzAesEntry) == 24
+ST_NOPASSWD, ST_WRONGPASSWD, ST_AUTH = 11, 12, 13
+
+
 class Lib:
     _inst = None
 
@@ -91,6 +101,10 @@ class Lib:
         L.otz_deflate_fetch.argtypes = [vp, vp, vp, u64]
         L.otz_deflate_chunks.argtypes = [vp, vp, vp, vp, vp, C.c_uint32, C.POINTER(C.c_uint32)]
         L.otz_deflate_host.argtypes = [vp, vp, u64, vp, vp, vp, C.c_uint32, vp, u64, vp, vp, vp, vp, C.POINTER(u64)]
+        L.otz_aes_open.argtypes = [vp, vp, u64, vp, C.c_uint32, vp, C.c_uint32, vp, u64]
+        L.otz_aes_status.argtypes = [vp, vp]
+        L.otz_aes_times.argtypes = [vp] + [C.POINTER(C.c_float)] * 3
+        L.otz_aes_seal.argtypes = [vp, vp, u64, vp, C.c_uint32, vp, vp, C.c_uint32, vp, u64]
 
     @classmethod
     def get(cls) -> "Lib":
@@ -405,3 +419,36 @@ class Ctx:
             if r < 0:
                 self.lib.check(r, "otz_deflate_chunks")
         return first[:n], cnt[:n], cs[:tot], int(cb.value)
+
+    # -- WinZip AES (device-resident buffers; what tools/aes_bench.py times)
+    @staticmethod
+    def _passwords(passwords):
+        arr = (C.c_char_p * max(len(passwords), 1))(*[p if isinstance(p, bytes) else p.encode() for p in passwords])
+        return arr, len(passwords)
+
+    def aes_open(self, d_src, src_len: int, rows: np.ndarray, passwords, d_plain, plain_len: int):
+        """Asynchronous: KDF + CTR into the plaintext image, MAC on the side stream.  rows: AES_ENTRY_DTYPE."""
+        r = np.ascontiguousarray(rows, dtype=AES_ENTRY_DTYPE)
+        pw, n_pw = self._passwords(passwords)
+        self._aes_keep = (r, pw)
+        self.lib.check(self.L.otz_aes_open(self.h, d_src, src_len, r.ctypes.data_as(C.c_void_p), len(r), pw, n_pw, d_plain, plain_len),
+                       "otz_aes_open")
+
+    def aes_status(self, n: int) -> np.ndarray:
+        st = np.zeros(max(n, 1), dtype=np.int32)
+        self.lib.check(self.L.otz_aes_status(self.h, st.ctypes.data_as(C.c_void_p)), "otz_aes_status")
+        return st[:n]
+
+    def aes_times(self):
+        """-> (ms_kdf, ms_ctr, ms_mac) of the last aes_open"""
+        f = [C.c_float() for _ in range(3)]
+        self.lib.check(self.L.otz_aes_times(self.h, *[C.byref(x) for x in f]), "otz_aes_times")
+        return tuple(x.value for x in f)
+
+    def aes_seal(self, d_in, in_len: int, rows: np.ndarray, salts: bytes, passwords, d_out, out_len: int):
+        r = np.ascontiguousarray(rows, dtype=AES_ENTRY_DTYPE)
+        pw, n_pw = self._passwords(passwords)
+        sb = np.frombuffer(salts, dtype=np.uint8)
+        assert sb.size >= 16 * len(r)
+        self.lib.check(self.L.otz_aes_seal(self.h, d_in, in_len, r.ctypes.data_as(C.c_void_p), len(r), sb.ctypes.data_as(C.c_void_p),
+                                           pw, n_pw, d_out, out_len), "otz_aes_seal")

@@ -9,6 +9,7 @@ from .native import Lib
 
 ZIP_RDONLY, ZIP_CREATE, ZIP_EXCL, ZIP_TRUNCATE = 0, 1, 2, 8
 ZIP_CM_STORE, ZIP_CM_DEFLATE = 0, 8
+ZIP_EM_NONE, ZIP_EM_TRAD_PKWARE, ZIP_EM_AES_128, ZIP_EM_AES_192, ZIP_EM_AES_256 = 0, 1, 0x0101, 0x0102, 0x0103
 
 
 class ZipFileT(C.Structure):  # struct zip_file
@@ -61,6 +62,12 @@ class ZipApi:
         L.zip_set_file_compression.argtypes = [P(ZipT), C.c_uint64, C.c_int32, C.c_uint32]
         L.zip_file_replace.argtypes = [P(ZipT), C.c_uint64, C.c_void_p, C.c_int]
         L.otezip_method_from_string.argtypes = [C.c_char_p]
+        L.zip_set_default_password.argtypes = [P(ZipT), C.c_char_p]
+        L.zip_fopen_index_encrypted.restype = P(ZipFileT)
+        L.zip_fopen_index_encrypted.argtypes = [P(ZipT), C.c_uint64, C.c_int, C.c_char_p]
+        L.zip_file_set_encryption.argtypes = [P(ZipT), C.c_uint64, C.c_uint16, C.c_char_p]
+        L.zip_encryption_method_supported.argtypes = [C.c_uint16, C.c_int]
+        L.otezip_b200_entry_status.argtypes = [P(ZipT), C.c_uint64]
         self.verify_crc = C.c_int.in_dll(L, "otezip_verify_crc")
         self.ignore_zipbomb = C.c_int.in_dll(L, "otezip_ignore_zipbomb")
         try:
