@@ -9,7 +9,7 @@ CUH := $(wildcard $(CSRC)/*.cuh) include/otz_gpu.h
 HOST_C := $(wildcard $(CSRC)/host/*.c)
 HOST_O := $(HOST_C:.c=.o)
 
-all: $(LIB) oracle debug
+all: $(LIB) oracle debug d64enc
 
 $(CSRC)/otz_shim.o: $(CSRC)/otz_shim.cu $(CUH)
 	$(NVCC) $(NVFLAGS) -c -o $@ $< 2> $(CSRC)/ptxas.log || (cat $(CSRC)/ptxas.log; false)
@@ -28,9 +28,15 @@ $(DBGLIB): $(CSRC)/otz_shim_dbg.o $(HOST_O)
 	$(NVCC) $(ARCH) -shared -o $@ $^ -lcudart_static -lpthread -ldl -lrt
 debug: $(DBGLIB)
 
+# Deflate64 / DEFLATE encoder of the tests and tools/deflate64_bench.py (tests/deflate64.py loads it with ctypes)
+D64ENC := tools/libd64enc.so
+$(D64ENC): tools/d64enc.c
+	$(CC) -O2 -Wall -Wextra -std=c99 -fPIC -shared -o $@ $<
+
 oracle: $(LIB)
 	$(MAKE) -C oracle
 
 clean:
-	rm -f $(CSRC)/*.o $(CSRC)/host/*.o $(LIB) $(DBGLIB) $(CSRC)/ptxas.log $(CSRC)/ptxas_dbg.log
-.PHONY: all oracle clean debug
+	rm -f $(CSRC)/*.o $(CSRC)/host/*.o $(LIB) $(DBGLIB) $(D64ENC) $(CSRC)/ptxas.log $(CSRC)/ptxas_dbg.log
+d64enc: $(D64ENC)
+.PHONY: all oracle clean debug d64enc

@@ -50,7 +50,7 @@ extern "C" {
 #define OTZ_ST_LFH_SIG 2       /* LFH signature mismatch                          otezip.c:421-423 */
 #define OTZ_ST_DATA_RANGE 3    /* payload outside the image                       otezip.c:438-446 */
 #define OTZ_ST_ZIPBOMB 4       /* uncomp > comp*ratio+slack                       otezip.c:454-462 */
-#define OTZ_ST_METHOD 5        /* method not on the GPU path (only 0, 8, 93)      otezip.c:662-665 */
+#define OTZ_ST_METHOD 5        /* method not on the GPU path (only 0, 8, 9, 93)   otezip.c:662-665 */
 #define OTZ_ST_STORE_SIZE 6    /* STORE with comp != uncomp                       otezip.c:482-485 */
 #define OTZ_ST_DATA 7          /* corrupt stream (Z_DATA_ERROR class)             dec / zstd */
 #define OTZ_ST_TRUNCATED 8     /* input exhausted before the stream ended (Z_BUF_ERROR class) */
@@ -69,6 +69,9 @@ extern "C" {
 /* ---- compression methods on this path (src/include/otezip/config.h:28-35) ---- */
 #define OTZ_M_STORE 0
 #define OTZ_M_DEFLATE 8
+/* read path only: Deflate64 (PKWARE "enhanced deflate"), decoded by k_inflate<G, W, true>.  The reference rejects the
+ * method, so a stream that decodes carries OTZ_STF_REF_EOB as well (handed out only when ref_compat is 0). */
+#define OTZ_M_DEFLATE64 9
 #define OTZ_M_ZSTD 93
 /* write path only: or-ed into method[i], compression level 1 ("fastest": one match candidate per position instead of the
  * eight-way search at the start of every token; about 3x the speed at 0.85x the ratio on text) */
@@ -198,7 +201,8 @@ int otz_extract_produced(otz_ctx *ctx, otz_plan *plan, uint32_t *produced);
 /* DEFLATE streams of the run last collected with otz_extract_results that the lane-per-stream decoder
  * (k_inflate_tok/k_inflate_lz) declined and the warp-per-stream decoder (k_inflate) decoded instead:
  * error and short streams, stored blocks with payload, code sets beyond the fixed table budget.  Both decoders
- * implement dec:547-831 with identical results; this is a performance counter. */
+ * implement dec:547-831 with identical results; this is a performance counter.  Deflate64 streams always run on
+ * k_inflate and are not counted. */
 uint32_t otz_inflate_fallbacks(otz_ctx *ctx);
 
 /* ---- multi-GPU sharding (SURVEY.md §8e; the reference has no counterpart: entries are independent,

@@ -49,6 +49,16 @@ int otezip_ref_compat = 1;
 int otezip_write_data_descriptors = 0;
 int otezip_zstd_frames = 0;
 
+/* OTEZIP_REF_COMPAT=0 in the environment sets the initial value of otezip_ref_compat, so that a program that never touches
+ * the global (the otezip CLI) can extract what the reference rejects: Deflate64 entries, F1 streams, real Zstandard frames.
+ * Read once, when the library is loaded; a program that assigns the global later still wins. */
+__attribute__ ((constructor)) static void otezip_env_defaults(void) {
+	const char *e = getenv ("OTEZIP_REF_COMPAT");
+	if (e && *e) {
+		otezip_ref_compat = atoi (e) != 0;
+	}
+}
+
 /* ---- private archive state; `pub` must stay first: zip_t* == struct otz_archive* ---- */
 struct otz_window {               /* one decoded batch of consecutive entries */
 	struct otz_window *next;
@@ -401,7 +411,7 @@ static int load_central(struct otz_archive *a) {
 					const uint8_t *d = x + xo + 4;
 					const uint16_t ver = sz == 7 ? otezip_read_le16 (d) : 0, am = sz == 7 ? otezip_read_le16 (d + 5) : 0xFFFF;
 					if ((ver == 1 || ver == 2) && d[2] == 'A' && d[3] == 'E' && d[4] >= 1 && d[4] <= 3 &&
-						(am == OTEZIP_METHOD_STORE || am == OTEZIP_METHOD_DEFLATE || am == OTEZIP_METHOD_ZSTD)) {
+						(am == OTEZIP_METHOD_STORE || am == OTEZIP_METHOD_DEFLATE || am == OTZ_M_DEFLATE64 || am == OTEZIP_METHOD_ZSTD)) {
 						a->aes[i].vendor = ver;
 						a->aes[i].strength = d[4];
 						a->aes[i].method = am;
@@ -848,7 +858,7 @@ static int32_t host_precheck(const struct otz_archive *a, zip_uint64_t i, const 
 		if (inner_comp (a, i) != e->uncomp_size) {
 			return OTZ_ST_STORE_SIZE;
 		}
-	} else if (method != OTEZIP_METHOD_DEFLATE && method != OTEZIP_METHOD_ZSTD) {
+	} else if (method != OTEZIP_METHOD_DEFLATE && method != OTZ_M_DEFLATE64 && method != OTEZIP_METHOD_ZSTD) {
 		return OTZ_ST_METHOD;
 	}
 	if (x && !pw) {
@@ -1340,6 +1350,13 @@ int zip_set_default_password(zip_t *za, const char *password) {
 	a->default_pw = copy;
 	a->pw_gen++;   /* cached AES results belong to the old password */
 	return 0;
+}
+
+int zip_compression_method_supported(zip_int32_t method, int compress) {
+	if (method == ZIP_CM_STORE || method == ZIP_CM_DEFLATE || method == OTEZIP_METHOD_ZSTD) {
+		return 1;
+	}
+	return !compress && method == ZIP_CM_DEFLATE64;   /* Deflate64 is read, never written */
 }
 
 int zip_encryption_method_supported(zip_uint16_t method, int encode) {

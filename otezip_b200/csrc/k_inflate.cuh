@@ -20,6 +20,11 @@
 // (dec:811-816: Z_BUF_ERROR as soon as the last input byte has been loaded and the stream is not
 // finished — SURVEY.md F1) and reports it as the OTZ_STF_REF_EOB flag, so the host library can
 // reproduce the reference's accept/reject decision bit for bit.
+//
+// D64 = true instantiates the Deflate64 decoder (ZIP method 9, PKWARE's "enhanced deflate"; the tables of zlib's
+// contrib/infback9/inftree9.c): a 64 KiB window, length symbol 285 = base 3 + 16 extra bits (lengths 3..65,538),
+// distance symbols 30 / 31 = base 32,769 / 49,153 + 14 extra bits, HDIST up to 32.  Everything else is shared; the
+// D64 = false instantiations are the DEFLATE decoder unchanged.
 #pragma once
 #include "otz_common.cuh"
 #include "k_copy.cuh"
@@ -40,6 +45,12 @@
 #define INF_ENTRY(cb, xb, kind, value) ((uint32_t)(cb) | ((uint32_t)(xb) << 5) | ((uint32_t)(kind) << 9) | ((uint32_t)(value) << 16))
 #define INF_INVALID INF_ENTRY(0u, 0u, INF_K_LINK, 0u)
 #define INF_KIND(e) (((e) >> 9) & 3u)
+// Deflate64 only: bit 11 adds 16 to the extra-bit count ([8:5] holds 0..15; symbol 285 needs 16)
+#define INF_XB16 (1u << 11)
+template <bool D64>
+__device__ __forceinline__ uint32_t inf_extra_bits(uint32_t e) {
+	return D64 ? ((e >> 5) & 15u) | ((e >> 7) & 16u) : (e >> 5) & 15u;
+}
 
 struct __align__(16) InflateSmem {
 	uint32_t lit[INF_LIT_CAP];
@@ -121,9 +132,10 @@ struct BitReader {
 };
 
 // Table entry of symbol s whose code takes cb bits at this table level.
+template <bool D64>
 __device__ __forceinline__ uint32_t inf_symbol_entry(uint32_t s, uint32_t cb, bool is_dist) {
 	if (is_dist) {
-		if (s >= 30) {
+		if (s >= 30 && !D64) {
 			return INF_INVALID;  // fixed-table symbols 30/31 (dec:766-774 would index past dist_base)
 		}
 		if (s < 4) {
@@ -146,7 +158,7 @@ __device__ __forceinline__ uint32_t inf_symbol_entry(uint32_t s, uint32_t cb, bo
 		return INF_ENTRY(cb, 0u, INF_K_LEN, 3u + v);
 	}
 	if (v == 28) {
-		return INF_ENTRY(cb, 0u, INF_K_LEN, 258u);
+		return D64 ? INF_ENTRY(cb, 0u, INF_K_LEN, 3u) | INF_XB16 : INF_ENTRY(cb, 0u, INF_K_LEN, 258u);
 	}
 	const uint32_t xb = (v - 4) >> 2;
 	return INF_ENTRY(cb, xb, INF_K_LEN, 3u + ((4u + (v & 3u)) << xb));  // dec:720-725
@@ -155,7 +167,7 @@ __device__ __forceinline__ uint32_t inf_symbol_entry(uint32_t s, uint32_t cb, bo
 // ------------------------------------------------------------------------------------------------
 // Canonical table build from code lengths (dec:86-119 assigns the same canonical codes).
 // Returns 0 ok, nonzero = invalid set.  All lanes return the same value.
-template <int G, typename Tile>
+template <int G, bool D64, typename Tile>
 __device__ __noinline__ int build_table(const Tile &tile, InflateSmem &S, const uint8_t *lens, int n, int root, uint32_t *tbl, int cap,
 	bool is_dist) {
 	const int lane = tile.thread_rank();
@@ -236,7 +248,7 @@ __device__ __noinline__ int build_table(const Tile &tile, InflateSmem &S, const 
 		}
 		const uint32_t c = S.first[l] + (i - S.offs[l]);
 		const uint32_t rev = __brev(c) >> (32 - l);
-		const uint32_t e = inf_symbol_entry(s, l, is_dist);
+		const uint32_t e = inf_symbol_entry<D64>(s, l, is_dist);
 		for (int k = (int)rev; k < rootsz; k += (1 << l)) {
 			tbl[k] = e;
 		}
@@ -275,7 +287,7 @@ __device__ __noinline__ int build_table(const Tile &tile, InflateSmem &S, const 
 				}
 			}
 			const uint32_t nb2 = (uint32_t)(l - root);
-			const uint32_t e = inf_symbol_entry(s, nb2, is_dist);
+			const uint32_t e = inf_symbol_entry<D64>(s, nb2, is_dist);
 			const int step = 1 << nb2;
 			for (int k = (int)(rev >> root) + lane * step; k < (1 << sub_bits); k += G * step) {
 				tbl[sub_off + k] = e;
@@ -287,28 +299,28 @@ __device__ __noinline__ int build_table(const Tile &tile, InflateSmem &S, const 
 }
 
 // dec:322-349
-template <int G, typename Tile>
+template <int G, bool D64, typename Tile>
 __device__ __noinline__ int build_fixed(const Tile &tile, InflateSmem &S) {
 	const int lane = tile.thread_rank();
 	for (int i = lane; i < 320; i += G) {
 		S.lens[i] = i < 144 ? 8 : i < 256 ? 9 : i < 280 ? 7 : i < 288 ? 8 : 5;
 	}
 	tile.sync();
-	int r = build_table<G>(tile, S, S.lens, 288, INF_LIT_ROOT, S.lit, INF_LIT_CAP, false);
-	r |= build_table<G>(tile, S, S.lens + 288, 32, INF_DST_ROOT, S.dst, INF_DST_CAP, true);
+	int r = build_table<G, D64>(tile, S, S.lens, 288, INF_LIT_ROOT, S.lit, INF_LIT_CAP, false);
+	r |= build_table<G, D64>(tile, S, S.lens + 288, 32, INF_DST_ROOT, S.dst, INF_DST_CAP, true);
 	return r;
 }
 
 // dec:122-266
-template <int G, typename Tile>
+template <int G, bool D64, typename Tile>
 __device__ __forceinline__ int read_dynamic(const Tile &tile, InflateSmem &S, BitReader<G> &br) {
 	const int lane = tile.thread_rank();
 	br.norm(tile);
 	uint32_t bits = br.peek();
 	const int hlit = (int)(bits & 31) + 257, hdist = (int)((bits >> 5) & 31) + 1, hclen = (int)((bits >> 10) & 15) + 4;
 	br.skip(14);
-	if (hlit > 286 || hdist > 30) {
-		return 1;  // RFC 1951 limits; dec:165-168 would overflow its scratch instead
+	if (hlit > 286 || (!D64 && hdist > 30)) {
+		return 1;  // RFC 1951 limits; dec:165-168 would overflow its scratch instead (Deflate64: HDIST up to 32, lens[] holds 286 + 32)
 	}
 	for (int i = lane; i < 19; i += G) {
 		S.lens[i] = 0;
@@ -404,11 +416,11 @@ __device__ __forceinline__ int read_dynamic(const Tile &tile, InflateSmem &S, Bi
 	if (S.lens[256] == 0) {
 		return 1;  // no end-of-block code
 	}
-	int r = build_table<G>(tile, S, S.lens, hlit, INF_LIT_ROOT, S.lit, INF_LIT_CAP, false);
+	int r = build_table<G, D64>(tile, S, S.lens, hlit, INF_LIT_ROOT, S.lit, INF_LIT_CAP, false);
 	if (r) {
 		return r;
 	}
-	return build_table<G>(tile, S, S.lens + hlit, hdist, INF_DST_ROOT, S.dst, INF_DST_CAP, true);
+	return build_table<G, D64>(tile, S, S.lens + hlit, hdist, INF_DST_ROOT, S.dst, INF_DST_CAP, true);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -479,9 +491,41 @@ struct OutRing {
 	}
 };
 
+// LZ77 copy of length <= 258 bytes from `dist` bytes back to linear position dq (whole tile; dist already validated).
+template <int G, int W, typename Tile>
+__device__ __forceinline__ void inf_copy(const Tile &tile, const OutRing<G, W> &ring, uint8_t *rb, uint32_t dq, uint32_t dist, uint32_t length,
+	int lane) {
+	constexpr uint32_t MASK = W - 1;
+	tile.sync();  // earlier ring stores of this tile are visible to the loads below
+	if (dist + length <= (uint32_t)W) {
+		const uint32_t sq = dq - dist;
+		if (dist >= length) {
+			for (uint32_t i = lane; i < length; i += G) {
+				rb[(dq + i) & MASK] = rb[(sq + i) & MASK];
+			}
+		} else {
+			// overlapping copy = periodic extension of the last `dist` bytes (dec:521-533)
+			uint32_t r = dist > (uint32_t)lane ? (uint32_t)lane : (uint32_t)lane % dist;
+			const uint32_t step = dist > (uint32_t)G ? (uint32_t)G : (uint32_t)G % dist;
+			for (uint32_t i = lane; i < length; i += G) {
+				rb[(dq + i) & MASK] = rb[(sq + r) & MASK];
+				r += step;
+				r = r >= dist ? r - dist : r;
+			}
+		}
+	} else {
+		// far back-reference: the source left the ring and is in HBM already (dist > W - 258 >= length)
+		const uint8_t *sp = ring.gbase + (dq - dist);
+		for (uint32_t i = lane; i < length; i += G) {
+			rb[(dq + i) & MASK] = sp[i];
+		}
+	}
+}
+
 // One literal / end-of-block / length+distance step (dec:662-799).  CHECKED adds the tests that only matter
-// near the end of the input or of the output buffer.  Returns 0 = continue, 1 = end of block, <0 = -status.
-template <int G, int W, bool CHECKED, typename Tile>
+// near the end of the input or of the output buffer.  Returns 0 = continue, 1 = end of block, <0 = -status;
+// Deflate64 only: 2 = a match longer than 258 bytes was executed (the caller's byte budget no longer holds).
+template <int G, int W, bool CHECKED, bool D64, typename Tile>
 __device__ __forceinline__ int inflate_event(const Tile &tile, const InflateSmem &S, BitReader<G> &br, OutRing<G, W> &ring, uint8_t *rb,
 	uint32_t qcap, int lane) {
 	constexpr uint32_t MASK = W - 1;
@@ -514,7 +558,7 @@ __device__ __forceinline__ int inflate_event(const Tile &tile, const InflateSmem
 		return 1;  // dec:711-716
 	}
 	// length (dec:720-737), then distance (dec:740-782)
-	const uint32_t xb = (e >> 5) & 15u;
+	const uint32_t xb = inf_extra_bits<D64>(e);   // cb + xb <= 15 + 16: within the 32 peeked bits
 	const uint32_t length = (e >> 16) + ((bits >> cb) & ((1u << xb) - 1u));
 	br.skip(cb + xb);
 	br.norm(tile);
@@ -541,36 +585,36 @@ __device__ __forceinline__ int inflate_event(const Tile &tile, const InflateSmem
 	if (CHECKED && length > qcap - dq) {
 		return -OTZ_ST_OVERFLOW;  // dec:535-541, :791-793
 	}
-	tile.sync();  // earlier ring stores of this tile are visible to the loads below
-	if (dist + length <= (uint32_t)W) {
-		const uint32_t sq = dq - dist;
-		if (dist >= length) {
-			for (uint32_t i = lane; i < length; i += G) {
-				rb[(dq + i) & MASK] = rb[(sq + i) & MASK];
-			}
-		} else {
-			// overlapping copy = periodic extension of the last `dist` bytes (dec:521-533)
-			uint32_t r = dist > (uint32_t)lane ? (uint32_t)lane : (uint32_t)lane % dist;
-			const uint32_t step = dist > (uint32_t)G ? (uint32_t)G : (uint32_t)G % dist;
-			for (uint32_t i = lane; i < length; i += G) {
-				rb[(dq + i) & MASK] = rb[(sq + r) & MASK];
-				r += step;
-				r = r >= dist ? r - dist : r;
-			}
+	if (D64 && length > 258u) {
+		if (!CHECKED && length > qcap - dq) {
+			return -OTZ_ST_OVERFLOW;
 		}
-	} else {
-		// far back-reference: the source left the ring and is in HBM already (dist > W - 258 >= length)
-		const uint8_t *sp = ring.gbase + (dq - dist);
-		for (uint32_t i = lane; i < length; i += G) {
-			rb[(dq + i) & MASK] = sp[i];
+		// A match of length L at distance d is the same as consecutive matches of <= 258 bytes, all at distance d.  Running
+		// them as such, with the ring flush the event loop performs between events, keeps every invariant of the
+		// 258-byte copy: the ring holds the pieces, a far source is already in HBM, overlap is the periodic copy.
+		uint32_t q = dq, left = length;
+		for (;;) {
+			const uint32_t n = min(left, 258u);
+			OTZ_CHK(q + n <= qcap, OTZ_CK_D64_OUT);
+			OTZ_CHK(q - dist >= ring.mis && (dist + n <= (uint32_t)W || q - dist + n <= ring.qf), OTZ_CK_D64_SRC);
+			inf_copy<G, W>(tile, ring, rb, q, dist, n, lane);
+			q += n;
+			left -= n;
+			ring.q = q;
+			if (!left) {
+				break;
+			}
+			ring.maybe_flush(tile, lane);
 		}
+		return CHECKED ? 0 : 2;
 	}
+	inf_copy<G, W>(tile, ring, rb, dq, dist, length, lane);
 	ring.q = dq + length;
 	return 0;
 }
 
 // Decode one raw stream.  Returns the status word; *produced = bytes written.
-template <int G, int W, typename Tile>
+template <int G, int W, bool D64, typename Tile>
 __device__ __forceinline__ int32_t inflate_stream(const Tile &tile, InflateSmemV2<G, W> &SS, const uint8_t *__restrict__ in, uint32_t comp,
 	uint8_t *__restrict__ out, uint32_t cap, uint32_t *produced, uint32_t row_flags) {
 	const int lane = tile.thread_rank();
@@ -663,13 +707,14 @@ __device__ __forceinline__ int32_t inflate_stream(const Tile &tile, InflateSmemV
 			err = OTZ_ST_DATA;  // dec:657-658
 			break;
 		}
-		if ((btype == 1 ? build_fixed<G>(tile, S) : read_dynamic<G>(tile, S, br)) != 0) {
+		if ((btype == 1 ? build_fixed<G, D64>(tile, S) : read_dynamic<G, D64>(tile, S, br)) != 0) {
 			err = OTZ_ST_DATA;
 			break;
 		}
 		INF_STEP_CHECK();
-		// ---- symbols.  An event consumes at most 48 bits (two window words) and produces at most 258 bytes, so
-		// `budget` events can run without any end-of-input / end-of-output test; the rest run one by one.
+		// ---- symbols.  An event consumes at most 48 bits (Deflate64: 60; two window words) and produces at most 258 bytes, so
+		// `budget` events can run without any end-of-input / end-of-output test; the rest run one by one.  (A longer Deflate64
+		// match tests the end of the output itself and ends the run of unchecked events.)
 		bool eob = false;
 		for (;;) {
 			int64_t budget = min(((int64_t)br.words_left - 2) >> 1, (int64_t)((qcap - ring.q) / 258u));
@@ -677,15 +722,19 @@ __device__ __forceinline__ int32_t inflate_stream(const Tile &tile, InflateSmemV
 			int rc = 0;
 			for (int32_t n = (int32_t)budget; n > 0; n--) {
 				br.norm(tile);
-				rc = inflate_event<G, W, false>(tile, S, br, ring, rb, qcap, lane);
+				rc = inflate_event<G, W, false, D64>(tile, S, br, ring, rb, qcap, lane);
 				if (rc) {
 					break;
 				}
 				ring.maybe_flush(tile, lane);
 			}
+			if (D64 && rc == 2) {
+				ring.maybe_flush(tile, lane);
+				continue;   // a long match used up an unknown part of the byte budget: compute it again
+			}
 			if (rc == 0 && budget <= 0) {
 				br.norm(tile);
-				rc = inflate_event<G, W, true>(tile, S, br, ring, rb, qcap, lane);
+				rc = inflate_event<G, W, true, D64>(tile, S, br, ring, rb, qcap, lane);
 				if (rc == 0) {
 					ring.maybe_flush(tile, lane);
 					INF_STEP_CHECK();
@@ -732,7 +781,7 @@ __device__ __forceinline__ int32_t inflate_stream(const Tile &tile, InflateSmemV
 
 // grid: persistent; each tile pulls the next entry of `list` (largest first) from a global counter.
 // n_list_dev != NULL: the list length lives in device memory (written by an earlier kernel of the same stream).
-template <int G, int W>
+template <int G, int W, bool D64 = false>
 __global__ void __launch_bounds__(256) k_inflate(const uint8_t *__restrict__ archive, uint8_t *__restrict__ out,
 	const otz_entry *__restrict__ ents, const OtzEntryState *__restrict__ est, int32_t *__restrict__ status,
 	const uint32_t *__restrict__ list, uint32_t n_list, uint32_t *__restrict__ work_counter, uint32_t *__restrict__ produced_out,
@@ -760,7 +809,10 @@ __global__ void __launch_bounds__(256) k_inflate(const uint8_t *__restrict__ arc
 		const otz_entry e = ents[ei];
 		uint8_t *dst = out + e.out_ofs;
 		uint32_t produced = 0;
-		int32_t st = inflate_stream<G, W>(tile, S, archive + est[ei].data_ofs, e.comp_size, dst, e.uncomp_size, &produced, e.flags);
+		int32_t st = inflate_stream<G, W, D64>(tile, S, archive + est[ei].data_ofs, e.comp_size, dst, e.uncomp_size, &produced, e.flags);
+		if (D64 && OTZ_ST_CODE(st) == OTZ_ST_OK) {
+			st |= OTZ_STF_REF_EOB;   // a valid stream of a method the reference rejects (otezip.c:662-665)
+		}
 		if ((e.flags & OTZ_EF_CHUNK) && OTZ_ST_CODE(st) != OTZ_ST_OK && lane == 0) {
 			status[e.crc32] = OTZ_ST_DATA;   // a failing chunk fails its parent row (e.crc32 = parent row)
 		}

@@ -49,6 +49,8 @@ __device__ unsigned long long g_otz_violations[OTZ_CHK_SLOTS];
 #define OTZ_CK_AES_WORK 19      // k_aes_ctr / k_aes_mac: work-list or job index out of range
 #define OTZ_CK_AES_OUT 20       // k_aes_ctr: plaintext-image / ciphertext store outside the output buffer
 #define OTZ_CK_AES_IN 21        // k_aes_ctr: load outside the input buffer
+#define OTZ_CK_D64_OUT 22       // k_inflate<D64>: piece of a long match beyond the entry's output slice
+#define OTZ_CK_D64_SRC 23       // k_inflate<D64>: piece source neither in the ring nor flushed to HBM, or before the slice
 
 #define OTZ_SIG_LFH 0x04034b50u
 #define OTZ_MAX_PAYLOAD (2ull * 1024ull * 1024ull * 1024ull)  // otezip.c:102

@@ -77,6 +77,8 @@ struct otz_ctx {
 	uint64_t h_res_bytes;
 	uint64_t sym_limit;     // OTZ_SEG_SYM_LIMIT: cap of the symbol buffer in elements (tests: streams that do not fit are walked by one warp)
 	struct OtzAesRun *aes;  // device state of the last otz_aes_open / otz_aes_seal (created on first use)
+	cudaStream_t stream_d64[2];   // Deflate64 entries (large / small), beside the DEFLATE work of the same run
+	cudaEvent_t ev_d64_fork, ev_d64_join[2];
 };
 
 struct otz_plan {
@@ -103,6 +105,8 @@ struct otz_plan {
 	uint32_t *d_zstd_list, n_zstd;
 	OtzCrcChunk *d_zchunks;    // CRC chunks of the method-93 entries (reference containers and real Zstandard frames)
 	uint32_t n_zchunks;
+	uint32_t *d_d64_list, n_d64;   // Deflate64 entries (method 9), longest first; [0, n_d64_big) are the large ones
+	uint32_t n_d64_big;
 	uint64_t *d_ztok_ofs;      // two-phase Zstandard: token scratch offset of every method-93 list slot (+ end)
 	uint64_t ztok_bytes;
 	I2TokRes *d_ztokres;
@@ -221,6 +225,11 @@ extern "C" int otz_ctx_create(int device, otz_ctx **out) {
 	CK(cudaEventCreateWithFlags(&c->ev_join, cudaEventDisableTiming));
 	CK(cudaEventCreateWithFlags(&c->ev_join3, cudaEventDisableTiming));
 	CK(cudaEventCreateWithFlags(&c->ev_join4, cudaEventDisableTiming));
+	for (int k = 0; k < 2; k++) {
+		CK(cudaStreamCreateWithFlags(&c->stream_d64[k], cudaStreamNonBlocking));
+		CK(cudaEventCreateWithFlags(&c->ev_d64_join[k], cudaEventDisableTiming));
+	}
+	CK(cudaEventCreateWithFlags(&c->ev_d64_fork, cudaEventDisableTiming));
 	CK(cudaEventCreate(&c->ev0));
 	CK(cudaEventCreate(&c->ev1));
 	for (auto &slot : c->pev) {
@@ -293,6 +302,11 @@ extern "C" void otz_ctx_destroy(otz_ctx *c) {
 	cudaEventDestroy(c->ev_join);
 	cudaEventDestroy(c->ev_join3);
 	cudaEventDestroy(c->ev_join4);
+	cudaEventDestroy(c->ev_d64_fork);
+	for (int k = 0; k < 2; k++) {
+		cudaEventDestroy(c->ev_d64_join[k]);
+		cudaStreamDestroy(c->stream_d64[k]);
+	}
 	cudaStreamDestroy(c->stream4);
 	cudaStreamDestroy(c->stream3);
 	cudaStreamDestroy(c->stream2);
@@ -457,6 +471,7 @@ extern "C" void otz_plan_destroy(otz_ctx *c, otz_plan *p) {
 	cudaFree(p->d_fb_list);
 	cudaFree(p->d_zstd_list);
 	cudaFree(p->d_zchunks);
+	cudaFree(p->d_d64_list);
 	cudaFree(p->d_ztok_ofs);
 	cudaFree(p->d_ztokres);
 	cudaFree(p->d_counter);
@@ -486,7 +501,7 @@ extern "C" int otz_plan_create(otz_ctx *c, const otz_entry *ents, uint32_t n, co
 	}
 	// Work lists.  CRC chunks: STORE entries first (they are also the copy list), then the rest.
 	std::vector<OtzCrcChunk> chunks;
-	std::vector<uint32_t> infl, zst;
+	std::vector<uint32_t> infl, zst, d64;
 	uint64_t need = 0;
 	for (int pass = 0; pass < 2; pass++) {
 		for (uint32_t i = 0; i < n; i++) {
@@ -510,6 +525,8 @@ extern "C" int otz_plan_create(otz_ctx *c, const otz_entry *ents, uint32_t n, co
 			}
 		} else if (ents[i].method == OTZ_M_ZSTD) {
 			zst.push_back(i);
+		} else if (ents[i].method == OTZ_M_DEFLATE64 && !(ents[i].flags & OTZ_EF_CHUNK)) {
+			d64.push_back(i);   // never on the two-phase path: its 32-bit records hold neither 64 KiB distances nor long lengths
 		}
 		if (!(opts->verify_only && ents[i].method == OTZ_M_STORE)) {
 			need = std::max<uint64_t>(need, ents[i].out_ofs + ents[i].uncomp_size);
@@ -541,6 +558,16 @@ extern "C" int otz_plan_create(otz_ctx *c, const otz_entry *ents, uint32_t n, co
 		p->n_inflate_big += ents[i].uncomp_size >= big_bytes;
 		p->n_inflate_huge += is_huge(i);
 	}
+	// Deflate64: sized as the one-kernel DEFLATE dispatch sizes its launches (large entries first, longest first)
+	std::stable_sort(d64.begin(), d64.end(), [&](uint32_t a, uint32_t b) {
+		const bool ba = ents[a].uncomp_size >= big_bytes, bb = ents[b].uncomp_size >= big_bytes;
+		return ba != bb ? ba : ents[a].comp_size > ents[b].comp_size;
+	});
+	p->n_d64_big = 0;
+	for (uint32_t i : d64) {
+		p->n_d64_big += ents[i].uncomp_size >= big_bytes;
+	}
+	p->n_d64 = (uint32_t)d64.size();
 	p->n_chunks = (uint32_t)chunks.size();
 	p->n_inflate = (uint32_t)infl.size();
 	p->n_zstd = (uint32_t)zst.size();
@@ -585,7 +612,7 @@ extern "C" int otz_plan_create(otz_ctx *c, const otz_entry *ents, uint32_t n, co
 	}
 	if ((rc = upload(&p->d_ents, ev, c->stream)) || (rc = upload(&p->d_chunks, chunks, c->stream)) ||
 		(rc = upload(&p->d_inflate_list, infl, c->stream)) || (rc = upload(&p->d_zstd_list, zst, c->stream)) ||
-		(rc = upload(&p->d_zchunks, zchunks, c->stream))) {
+		(rc = upload(&p->d_zchunks, zchunks, c->stream)) || (rc = upload(&p->d_d64_list, d64, c->stream))) {
 		otz_plan_destroy(c, p);
 		return rc;
 	}
@@ -616,18 +643,18 @@ extern "C" int otz_plan_create(otz_ctx *c, const otz_entry *ents, uint32_t n, co
 	return OTZ_SUCCESS;
 }
 
-template <int G, int W>
+template <int G, int W, bool D64 = false>
 static int launch_inflate(otz_ctx *c, otz_plan *p, const uint8_t *d_archive, uint8_t *d_out, const uint32_t *d_list, uint32_t count,
 	uint32_t *d_work, cudaStream_t st, const uint32_t *d_count) {
 	const int threads = 8 * G;   // 8 streams per CTA
 	const size_t smem = 8 * sizeof(InflateSmemV2<G, W>);
 	static bool attr_done = false;
 	if (!attr_done) {
-		CK(cudaFuncSetAttribute(k_inflate<G, W>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+		CK(cudaFuncSetAttribute(k_inflate<G, W, D64>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
 		attr_done = true;
 	}
 	int per_sm = 0;
-	CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_inflate<G, W>, threads, smem));
+	CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_inflate<G, W, D64>, threads, smem));
 	if (per_sm < 1) {
 		snprintf(g_err, sizeof(g_err), "k_inflate<%d,%d> does not fit an SM (%zu bytes of shared memory)", G, W, smem);
 		return OTZ_ERR_CUDA;
@@ -636,21 +663,22 @@ static int launch_inflate(otz_ctx *c, otz_plan *p, const uint8_t *d_archive, uin
 	uint32_t grid = (uint32_t)(c->sm_count * per_sm);
 	const uint32_t want = (count + tiles_per_cta - 1) / tiles_per_cta;
 	grid = std::max(1u, std::min(grid, want));
-	k_inflate<G, W><<<grid, threads, smem, st>>>(d_archive, d_out, p->d_ents, p->d_est, p->d_status, d_list, count, d_work, p->d_produced, d_count);
+	k_inflate<G, W, D64><<<grid, threads, smem, st>>>(d_archive, d_out, p->d_ents, p->d_est, p->d_status, d_list, count, d_work, p->d_produced, d_count);
 	c->launches++;
 	CK(cudaGetLastError());
 	return OTZ_SUCCESS;
 }
 
+template <bool D64 = false>
 static int launch_inflate_cfg(otz_ctx *c, otz_plan *p, const uint8_t *d_archive, uint8_t *d_out, int g, int w, uint32_t first, uint32_t count,
 	int slot /* word of d_counter used as the work counter */, cudaStream_t st, const uint32_t *d_list = nullptr,
 	const uint32_t *d_count = nullptr) {
 	if (!d_list) {
-		d_list = p->d_inflate_list + first;
+		d_list = (D64 ? p->d_d64_list : p->d_inflate_list) + first;
 	}
 #define OTZ_INF_CASE(G_, W_)        \
 	if (g == G_ && w == W_) {       \
-		return launch_inflate<G_, W_>(c, p, d_archive, d_out, d_list, count, p->d_counter + slot, st, d_count); \
+		return launch_inflate<G_, W_, D64>(c, p, d_archive, d_out, d_list, count, p->d_counter + slot, st, d_count); \
 	}
 	OTZ_INF_CASE(32, 16384)
 	OTZ_INF_CASE(32, 4096)
@@ -1008,6 +1036,38 @@ static int dispatch_inflate(otz_ctx *c, otz_plan *p, const uint8_t *d_archive, u
 	return launch_inflate_cfg(c, p, d_archive, d_out, 32, 2048, 0, p->n_inflate, 0, c->stream);
 }
 
+// Deflate64 entries (k_inflate<G, W, true>): launched right behind k_resolve on streams of their own, so that they run next to
+// the DEFLATE and Zstandard work of the run; *joins = number of ev_d64_join events the main stream must wait for before the
+// CRC.  The launches are sized as dispatch_inflate's legacy branch sizes them; OTZ_INFLATE_TILE / OTZ_INFLATE_RING select one
+// instantiation for all of them.  Work counters: words 24 and 25 of d_counter, which no other launch uses.
+static int dispatch_deflate64(otz_ctx *c, otz_plan *p, const uint8_t *d_archive, uint8_t *d_out, int *joins) {
+	CK(cudaEventRecord(c->ev_d64_fork, c->stream));
+	int &used = *joins, rc = OTZ_SUCCESS;
+	used = 0;
+	auto launch = [&](int g, int w, uint32_t first, uint32_t count) {
+		cudaStream_t st = c->stream_d64[used];
+		CK(cudaStreamWaitEvent(st, c->ev_d64_fork, 0));
+		const int r = launch_inflate_cfg<true>(c, p, d_archive, d_out, g, w, first, count, 24 + used, st);
+		CK(cudaEventRecord(c->ev_d64_join[used], st));
+		used++;
+		return r;
+	};
+	const uint32_t n_big = p->n_d64_big, n_small = p->n_d64 - n_big;
+	if (c->inflate_tile || c->inflate_ring) {
+		rc = launch(c->inflate_tile ? c->inflate_tile : 32, c->inflate_ring ? c->inflate_ring : 2048, 0, p->n_d64);
+	} else if (n_small <= (uint32_t)c->sm_count * 10u) {
+		rc = launch(32, 16384, 0, p->n_d64);
+	} else {
+		if (n_big) {
+			rc = launch(32, 16384, 0, n_big);
+		}
+		if (rc == OTZ_SUCCESS) {
+			rc = launch(32, 2048, n_big, n_small);
+		}
+	}
+	return rc;
+}
+
 extern "C" int otz_extract_run(otz_ctx *c, otz_plan *p, const uint8_t *d_archive, uint64_t archive_len, uint8_t *d_out,
 	uint64_t out_len) {
 	if (!c || !p || (!d_archive && archive_len)) {
@@ -1033,6 +1093,13 @@ extern "C" int otz_extract_run(otz_ctx *c, otz_plan *p, const uint8_t *d_archive
 	}
 	if (c->profile) {
 		CK(cudaEventRecord(pev[1], s));
+	}
+	int d64_joins = 0;
+	if (p->n_d64) {
+		const int rc = dispatch_deflate64(c, p, d_archive, d_out, &d64_joins);
+		if (rc) {
+			return rc;
+		}
 	}
 	if (p->n_store_chunks && !p->opts.verify_only) {
 		k_store_copy<<<std::min((uint32_t)c->sm_count * 4, (p->n_store_chunks + 7) / 8), 256, 0, s>>>(d_archive, d_out, p->d_ents, p->d_est,
@@ -1127,6 +1194,9 @@ extern "C" int otz_extract_run(otz_ctx *c, otz_plan *p, const uint8_t *d_archive
 		if (rc) {
 			return rc;
 		}
+	}
+	for (int k = 0; k < d64_joins; k++) {
+		CK(cudaStreamWaitEvent(s, c->ev_d64_join[k], 0));
 	}
 	if (c->profile) {
 		CK(cudaEventRecord(pev[2], s));

@@ -8,7 +8,7 @@ import ctypes as C
 from .native import Lib
 
 ZIP_RDONLY, ZIP_CREATE, ZIP_EXCL, ZIP_TRUNCATE = 0, 1, 2, 8
-ZIP_CM_STORE, ZIP_CM_DEFLATE = 0, 8
+ZIP_CM_STORE, ZIP_CM_DEFLATE, ZIP_CM_DEFLATE64 = 0, 8, 9
 ZIP_EM_NONE, ZIP_EM_TRAD_PKWARE, ZIP_EM_AES_128, ZIP_EM_AES_192, ZIP_EM_AES_256 = 0, 1, 0x0101, 0x0102, 0x0103
 
 
@@ -67,6 +67,7 @@ class ZipApi:
         L.zip_fopen_index_encrypted.argtypes = [P(ZipT), C.c_uint64, C.c_int, C.c_char_p]
         L.zip_file_set_encryption.argtypes = [P(ZipT), C.c_uint64, C.c_uint16, C.c_char_p]
         L.zip_encryption_method_supported.argtypes = [C.c_uint16, C.c_int]
+        L.zip_compression_method_supported.argtypes = [C.c_int32, C.c_int]
         L.otezip_b200_entry_status.argtypes = [P(ZipT), C.c_uint64]
         self.verify_crc = C.c_int.in_dll(L, "otezip_verify_crc")
         self.ignore_zipbomb = C.c_int.in_dll(L, "otezip_ignore_zipbomb")
