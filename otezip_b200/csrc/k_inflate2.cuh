@@ -16,7 +16,7 @@
 //            batch k executes, batch k+1 has been scanned, the descriptor of every match sits in its lane's registers
 //            and the sources of its far matches (those that left the shared-memory ring) are on their way into a
 //            staging buffer behind the ring by cp.async — so executing a batch touches shared memory only; the
-//            matches run in stream order, one shuffle pair and up to 64 elements per step; completed 512-byte
+//            matches run in stream order, three shuffles and up to 64 elements per step; completed 512-byte
 //            segments leave as coalesced 16-byte stores.  The same kernel executes Zstandard sequences (8-byte
 //            records, k_zstd.cuh) and the segments of huge streams over 16-bit symbols (below).
 //
@@ -29,6 +29,7 @@
 #pragma once
 #include "otz_common.cuh"
 #include "k_inflate.cuh"
+#include <type_traits>
 
 #ifndef OTZ_BYTE_STAGE_VECS
 #define OTZ_BYTE_STAGE_VECS 64u
@@ -601,7 +602,7 @@ __device__ __forceinline__ void i2_flush_range(T *gbase, const T *ring, uint32_t
 
 // overlapping LZ77 copy (distance < length): periodic extension of the last `dd` bytes, whole warp (dec:521-533)
 template <int W, typename T>
-__device__ __noinline__ void i2_copy_periodic(T *rb, uint32_t dq, uint32_t sq, uint32_t dd, uint32_t len, uint32_t lane) {
+__device__ __forceinline__ void i2_copy_periodic(T *rb, uint32_t dq, uint32_t sq, uint32_t dd, uint32_t len, uint32_t lane) {
 	constexpr uint32_t MASK = W - 1;
 	uint32_t r = dd > lane ? lane : lane % dd;
 	const uint32_t step = dd > 32u ? 32u : 32u % dd;
@@ -614,6 +615,44 @@ __device__ __noinline__ void i2_copy_periodic(T *rb, uint32_t dq, uint32_t sq, u
 
 __device__ __forceinline__ uint32_t i2_ld_le16(const uint8_t *p) { return (uint32_t)p[0] | ((uint32_t)p[1] << 8); }
 
+// one element at shared-memory byte address sa + OFS, loaded into / stored from a 32-bit register by the lanes where
+// x < len (the predicate is formed in the same statement, so no register has to be zeroed or zero-extended)
+template <typename T, int OFS>
+__device__ __forceinline__ uint32_t i2_lds_lt(uint32_t sa, uint32_t x, uint32_t len) {
+	uint32_t v;
+	if (sizeof(T) == 1) {
+		asm volatile("{\n\t.reg .pred p;\n\tsetp.lt.u32 p, %1, %2;\n\t@p ld.shared.u8 %0, [%3+%4];\n\t}" : "=r"(v) : "r"(x), "r"(len), "r"(sa), "n"(OFS) : "memory");
+	} else {
+		asm volatile("{\n\t.reg .pred p;\n\tsetp.lt.u32 p, %1, %2;\n\t@p ld.shared.u16 %0, [%3+%4];\n\t}" : "=r"(v) : "r"(x), "r"(len), "r"(sa), "n"(OFS) : "memory");
+	}
+	return v;
+}
+template <typename T, int OFS>
+__device__ __forceinline__ void i2_sts_lt(uint32_t sa, uint32_t x, uint32_t len, uint32_t v) {
+	if (sizeof(T) == 1) {
+		asm volatile("{\n\t.reg .pred p;\n\tsetp.lt.u32 p, %0, %1;\n\t@p st.shared.u8 [%2+%3], %4;\n\t}" ::"r"(x), "r"(len), "r"(sa), "n"(OFS), "r"(v) : "memory");
+	} else {
+		asm volatile("{\n\t.reg .pred p;\n\tsetp.lt.u32 p, %0, %1;\n\t@p st.shared.u16 [%2+%3], %4;\n\t}" ::"r"(x), "r"(len), "r"(sa), "n"(OFS), "r"(v) : "memory");
+	}
+}
+
+// a match of the common case (at most 64 elements, no overlap, neither range wraps around the ring): lane copies
+// elements lane and lane + 32.  ring_sa: the ring's shared-memory byte address; d, s: those of element 0 of the
+// destination (a ring slot) and of the source (ring or staging buffer, one index space: ring_sa + element index * sizeof(T))
+template <int W, typename T>
+__device__ __forceinline__ void i2_chk_simple(uint32_t ring_sa, uint32_t len, uint32_t d, uint32_t s) {
+	constexpr uint32_t RING = W * sizeof(T), ALL = (W + 2u * I2Elem<T>::STAGE) * sizeof(T);
+	const uint32_t dq = d - ring_sa, sq = s - ring_sa, n = len * (uint32_t)sizeof(T);
+	OTZ_CHK(len == 0u || (dq + n <= RING && sq + n <= ALL && (sq >= RING || sq + n <= RING)), len && dq + n > RING ? OTZ_CK_LZ_RING_DST : OTZ_CK_LZ_RING_SRC);
+}
+template <typename T>
+__device__ __forceinline__ void i2_copy_simple(uint32_t d, uint32_t s, uint32_t len, uint32_t lane) {
+	// (d, s: addresses of element `lane`)
+	const uint32_t v0 = i2_lds_lt<T, 0>(s, lane, len), v1 = i2_lds_lt<T, 32 * sizeof(T)>(s, lane + 32u, len);
+	i2_sts_lt<T, 0>(d, lane, len, v0);
+	i2_sts_lt<T, 32 * sizeof(T)>(d, lane + 32u, len, v1);
+}
+
 // what the scan of one batch leaves in registers for its execution
 struct I2Batch {
 	uint32_t ntake;     // records in the batch (0 = none left)
@@ -624,14 +663,19 @@ struct I2Batch {
 	uint32_t my_out;    //   its linear output position
 	uint32_t lit4;      //   and its first four literal bytes
 	// the match of this lane's record, as the executor wants it (it walks the records in stream order and fetches
-	// these two words with one shuffle each):
-	uint32_t ma;        //   ring index of the destination | length << 16 | I2_MF_* << 28 | bit 31 = any flag   (length 0: no match)
-	uint32_t mb;        //   source, as an element index from the ring's base: a ring index (< W), or an index into the staging
-	                    //   buffer behind the ring (>= W: a FAR source, fetched while the batch before ran)
-	uint32_t m_dist;    //   distance (overlapping matches are extended periodically)
+	// these three words with one shuffle each):
+	uint32_t mlen;      //   length | I2_MF_* flags above it: <= I2_ML_SIMPLE exactly when the match is the common case
+	                    //   (length 0: no match)
+	uint32_t mdst;      //   shared-memory byte address of the destination's ring slot
+	uint32_t msrc;      //   shared-memory byte address of the source: a ring slot, or a slot of the staging buffer behind the
+	                    //   ring (a FAR source, fetched while the batch before ran)
+	uint32_t spec;      // warp-uniform: bit r set when record r is not the common case (mlen > I2_ML_SIMPLE)
 };
-#define I2_MF_LONG 1u       // longer than 64 elements, or a range that wraps around the ring
-#define I2_MF_PERIODIC 2u   // distance < length
+#define I2_ML_LEN 0x1FFu          // mlen: the length
+#define I2_ML_SIMPLE 64u          // at most 64 elements and no flag: two loads and two stores per lane, nothing else
+#define I2_MF_DEP (1u << 9)       // the source reaches into what this batch itself writes
+#define I2_MF_LONG (1u << 10)     // longer than 64 elements, or a range that wraps around the ring
+#define I2_MF_PERIODIC (1u << 11) // distance < length
 
 // scan records [b, b + 32) (this lane holds record b + lane in `rec`): positions by warp prefix sums, the match descriptor
 // of every record (kept in its lane), and the copies of the batch's far sources into staging buffer `buf` are started.
@@ -681,8 +725,7 @@ __device__ __forceinline__ I2Batch i2_scan_batch(I2LzSmem<W, T> &S, int buf, uin
 	const bool is_far = is_match && dist > (uint32_t)W - (B.q_end - mq);
 	const uint32_t far_m = __ballot_sync(0xFFFFFFFFu, is_far);
 	const uint32_t src_lin = mq - dist;
-	B.mb = src_lin & MASK;
-	B.m_dist = dist;
+	uint32_t mb = src_lin & MASK;   // the source as an element index from the ring's base (>= W: staging buffer)
 	bool taken = mine;
 	if (far_m) {
 		// staging vectors per far match (the source is copied as whole 16-byte vectors)
@@ -713,7 +756,7 @@ __device__ __forceinline__ I2Batch i2_scan_batch(I2LzSmem<W, T> &S, int buf, uin
 		if (is_far && taken) {
 			const uint32_t cst = incl - nch;
 			OTZ_CHK(VEC * cst + soff + ml <= I2Elem<T>::STAGE, OTZ_CK_LZ_STAGE);
-			B.mb = (uint32_t)W + (uint32_t)buf * I2Elem<T>::STAGE + VEC * cst + soff;
+			mb = (uint32_t)W + (uint32_t)buf * I2Elem<T>::STAGE + VEC * cst + soff;
 			// every lane fetches the vectors of its own match (cp.async groups are per thread: the executor waits for
 			// its own group and then syncs the warp)
 			uint32_t sa = (uint32_t)__cvta_generic_to_shared(&S.stage[buf][VEC * cst]);
@@ -730,12 +773,16 @@ __device__ __forceinline__ I2Batch i2_scan_batch(I2LzSmem<W, T> &S, int buf, uin
 	// LONG: more than 64 elements, or the destination / a ring source wraps around the ring
 	const uint32_t flags = has_match ? (((ml > 64u || (mq & MASK) + ml > (uint32_t)W || (!is_far && (src_lin & MASK) + ml > (uint32_t)W)) ? I2_MF_LONG : 0u) |
 		((!is_far && dist < ml) ? I2_MF_PERIODIC : 0u)) : 0u;
-	// bit 27: the source reaches into what this batch itself writes (earlier matches, its literal runs), so the executor has
+	// DEP: the source reaches into what this batch itself writes (earlier matches, its literal runs), so the executor has
 	// to make the stores before it visible first; every other match only reads older ring data or its staged source and
 	// runs back to back with its neighbours (no WAR either: a near source lies above q_end - W, a slot no store of this
 	// batch touches)
-	const uint32_t dep = (has_match && src_lin + ml > q) ? 0x08000000u : 0u;
-	B.ma = (mq & MASK) | ((has_match ? ml : 0u) << 16) | dep | (flags << 28) | (flags ? 0x80000000u : 0u);
+	const uint32_t dep = (has_match && src_lin + ml > q) ? I2_MF_DEP : 0u;
+	B.mlen = has_match ? ml | dep | flags : 0u;
+	const uint32_t ring_sa = (uint32_t)__cvta_generic_to_shared(S.ring);
+	B.mdst = ring_sa + (mq & MASK) * (uint32_t)sizeof(T);
+	B.msrc = ring_sa + mb * (uint32_t)sizeof(T);
+	B.spec = __ballot_sync(0xFFFFFFFFu, B.mlen > I2_ML_SIMPLE);
 	asm volatile("cp.async.commit_group;" ::: "memory");
 	return B;
 }
@@ -743,10 +790,12 @@ __device__ __forceinline__ I2Batch i2_scan_batch(I2LzSmem<W, T> &S, int buf, uin
 // SEG: `list` holds huge streams; the tokens of a stream are the chain of segments k_seg_stitch accepted, walked by
 // this warp.  PAR: the work items are single segments of such chains (seg.par_items), executed over 16-bit symbols
 // into the symbol buffer `out` with the 32 KiB before the segment standing in as MARKERS (k_seg_window resolves them).
-template <int W, bool WIDE, bool SEG, bool PAR = false>
-__global__ void __launch_bounds__(128) k_inflate_lz(uint8_t *__restrict__ out, const otz_entry *__restrict__ ents, const uint32_t *__restrict__ list,
-	uint32_t n_list, uint32_t *__restrict__ work_counter, const uint8_t *__restrict__ scratch, const uint64_t *__restrict__ tok_ofs,
-	const I2TokRes *__restrict__ tokres, int32_t *__restrict__ status, uint32_t *__restrict__ produced_out, I2SegCtl seg, uint32_t k_first) {
+#define I2_LZ_PARAMS uint8_t *__restrict__ out, const otz_entry *__restrict__ ents, const uint32_t *__restrict__ list, uint32_t n_list, \
+	uint32_t *__restrict__ work_counter, const uint8_t *__restrict__ scratch, const uint64_t *__restrict__ tok_ofs, \
+	const I2TokRes *__restrict__ tokres, int32_t *__restrict__ status, uint32_t *__restrict__ produced_out, I2SegCtl seg, uint32_t k_first
+#define I2_LZ_ARGS out, ents, list, n_list, work_counter, scratch, tok_ofs, tokres, status, produced_out, seg, k_first
+template <int W, bool WIDE, bool SEG, bool PAR>
+__device__ __forceinline__ void i2_inflate_lz(I2_LZ_PARAMS) {
 	typedef typename I2ElemOf<PAR>::type T;
 	static_assert(!PAR || (SEG && !WIDE), "PAR executes segments of DEFLATE streams");
 	extern __shared__ __align__(16) uint8_t smem_raw[];
@@ -754,6 +803,8 @@ __global__ void __launch_bounds__(128) k_inflate_lz(uint8_t *__restrict__ out, c
 	const uint32_t lane = threadIdx.x & 31u;
 	I2LzSmem<W, T> &S = reinterpret_cast<I2LzSmem<W, T> *>(smem_raw)[threadIdx.x >> 5];
 	T *const rb = S.ring;
+	// the ring's shared-memory byte address, and this lane's byte offset within a match's first 32 elements
+	const uint32_t ring_sa = (uint32_t)__cvta_generic_to_shared(rb), lo = lane * (uint32_t)sizeof(T), lane32 = lane + 32u;
 	if (PAR) {
 		n_list = *seg.n_par;
 	}
@@ -883,44 +934,55 @@ __global__ void __launch_bounds__(128) k_inflate_lz(uint8_t *__restrict__ out, c
 						rb[(cur.my_out + t) & MASK] = lits[cur.my_lit + t];
 					}
 				}
-				// the matches in stream order: one shuffle pair fetches the record's descriptor; the common case — up to 64 elements,
-				// no overlap, neither range wraps around the ring — is two loads and two stores per lane without any index masking
-				// (source: ring or staging buffer, one index space); everything else takes the side exit
-				const uint32_t lane32 = lane + 32u;
-				// (the descriptor of record r + 1 is fetched while record r is executed: the shuffles are off the critical path)
-				uint32_t a_nx = __shfl_sync(0xFFFFFFFFu, cur.ma, 0), b_nx = __shfl_sync(0xFFFFFFFFu, cur.mb, 0);
+				// the matches in stream order: three shuffles fetch a record's descriptor.  The common case — up to 64 elements, no
+				// overlap, neither range wraps around the ring, no dependency on this batch's stores — is two loads and two stores
+				// per lane at addresses the scan resolved.  Such records run back to back in pairs, the loads of both before their
+				// stores (neither reads what the other writes, see DEP); the warp-uniform mask `spec` cuts the batch into runs of
+				// them, and the record behind each run takes the side path.
 #pragma unroll 1
-				for (uint32_t r = 0; r < cur.ntake; r++) {
-					const uint32_t a = a_nx, bsrc = b_nx;
-					a_nx = __shfl_sync(0xFFFFFFFFu, cur.ma, r + 1u);
-					b_nx = __shfl_sync(0xFFFFFFFFu, cur.mb, r + 1u);
-					if (a & 0x88000000u) {
-						__syncwarp();   // earlier ring stores of this batch are visible to the loads below (side exits: always)
+				for (uint32_t r = 0, spec = cur.spec;; r++, spec &= spec - 1u) {
+					const uint32_t end = spec ? (uint32_t)__ffs(spec) - 1u : cur.ntake;
+#pragma unroll 1
+					for (; r + 1u < end; r += 2u) {
+						const uint32_t la = __shfl_sync(0xFFFFFFFFu, cur.mlen, r), lb = __shfl_sync(0xFFFFFFFFu, cur.mlen, r + 1u);
+						const uint32_t da = __shfl_sync(0xFFFFFFFFu, cur.mdst, r), db = __shfl_sync(0xFFFFFFFFu, cur.mdst, r + 1u);
+						const uint32_t sa = __shfl_sync(0xFFFFFFFFu, cur.msrc, r), sb = __shfl_sync(0xFFFFFFFFu, cur.msrc, r + 1u);
+						i2_chk_simple<W, T>(ring_sa, la, da, sa);
+						i2_chk_simple<W, T>(ring_sa, lb, db, sb);
+						const uint32_t a0 = i2_lds_lt<T, 0>(sa + lo, lane, la), a1 = i2_lds_lt<T, 32 * sizeof(T)>(sa + lo, lane32, la);
+						const uint32_t b0 = i2_lds_lt<T, 0>(sb + lo, lane, lb), b1 = i2_lds_lt<T, 32 * sizeof(T)>(sb + lo, lane32, lb);
+						i2_sts_lt<T, 0>(da + lo, lane, la, a0);
+						i2_sts_lt<T, 32 * sizeof(T)>(da + lo, lane32, la, a1);
+						i2_sts_lt<T, 0>(db + lo, lane, lb, b0);
+						i2_sts_lt<T, 32 * sizeof(T)>(db + lo, lane32, lb, b1);
 					}
-					if ((int32_t)a >= 0) {
-						const uint32_t len = (a >> 16) & 0x1FFu, dq = a & 0xFFFFu;
-						T v0 = 0, v1 = 0;
-						OTZ_CHK(len == 0u || (dq + len <= (uint32_t)W && bsrc + len <= (uint32_t)W + 2u * I2Elem<T>::STAGE && (bsrc >= (uint32_t)W || bsrc + len <= (uint32_t)W)),
-							len && dq + len > (uint32_t)W ? OTZ_CK_LZ_RING_DST : OTZ_CK_LZ_RING_SRC);
-						if (lane < len) {
-							v0 = rb[bsrc + lane];
-						}
-						if (lane32 < len) {
-							v1 = rb[bsrc + lane32];
-						}
-						if (lane < len) {
-							rb[dq + lane] = v0;
-						}
-						if (lane32 < len) {
-							rb[dq + lane32] = v1;
-						}
+					if (r < end) {
+						const uint32_t l = __shfl_sync(0xFFFFFFFFu, cur.mlen, r), d = __shfl_sync(0xFFFFFFFFu, cur.mdst, r),
+							s = __shfl_sync(0xFFFFFFFFu, cur.msrc, r);
+						i2_chk_simple<W, T>(ring_sa, l, d, s);
+						i2_copy_simple<T>(d + lo, s + lo, l, lane);
+						r++;
+					}
+					if (!spec) {
+						break;
+					}
+					// record r: the side path
+					const uint32_t ml = __shfl_sync(0xFFFFFFFFu, cur.mlen, r), d = __shfl_sync(0xFFFFFFFFu, cur.mdst, r),
+						s = __shfl_sync(0xFFFFFFFFu, cur.msrc, r);
+					const uint32_t len = ml & I2_ML_LEN;
+					__syncwarp();   // earlier ring stores of this batch are visible to the loads below
+					if (ml < I2_MF_LONG) {
+						// DEP only: once those stores are visible, the common case
+						i2_chk_simple<W, T>(ring_sa, len, d, s);
+						i2_copy_simple<T>(d + lo, s + lo, len, lane);
 						continue;
 					}
-					const uint32_t len = (a >> 16) & 0x1FFu, dq = a & 0xFFFFu, fl = (a >> 28) & 7u;
-					const uint32_t smask = bsrc >= (uint32_t)W ? 0xFFFFFFFFu : MASK;   // staged sources are not wrapped
-					if (fl & I2_MF_PERIODIC) {
-						i2_copy_periodic<W, T>(rb, dq, bsrc, __shfl_sync(0xFFFFFFFFu, cur.m_dist, r), len, lane);
+					const uint32_t dq = (d - ring_sa) / (uint32_t)sizeof(T), bsrc = (s - ring_sa) / (uint32_t)sizeof(T);
+					if (ml & I2_MF_PERIODIC) {
+						// (a ring source below the destination: the distance is their distance around the ring)
+						i2_copy_periodic<W, T>(rb, dq, bsrc, (dq - bsrc) & MASK, len, lane);
 					} else {
+						const uint32_t smask = bsrc >= (uint32_t)W ? 0xFFFFFFFFu : MASK;   // staged sources are not wrapped
 #pragma unroll 1
 						for (uint32_t x = lane; x < len; x += 32) {
 							rb[(dq + x) & MASK] = rb[(bsrc + x) & smask];
@@ -970,4 +1032,15 @@ __global__ void __launch_bounds__(128) k_inflate_lz(uint8_t *__restrict__ out, c
 		}
 		__syncwarp();
 	}
+}
+
+// The chain walk (SEG, not PAR) keeps more state across its loops; its big ring leaves room for 3 CTAs an SM, and the
+// register budget that goes with it spares it a spill.  Every other instantiation keeps the compiler's own choice.
+template <int W, bool WIDE, bool SEG, bool PAR = false>
+__global__ typename std::enable_if<!SEG || PAR>::type __launch_bounds__(128) k_inflate_lz(I2_LZ_PARAMS) {
+	i2_inflate_lz<W, WIDE, SEG, PAR>(I2_LZ_ARGS);
+}
+template <int W, bool WIDE, bool SEG, bool PAR = false>
+__global__ typename std::enable_if<SEG && !PAR>::type __launch_bounds__(128, 3) k_inflate_lz(I2_LZ_PARAMS) {
+	i2_inflate_lz<W, WIDE, SEG, PAR>(I2_LZ_ARGS);
 }
