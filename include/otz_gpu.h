@@ -76,6 +76,10 @@ extern "C" {
 /* write path only: or-ed into method[i], compression level 1 ("fastest": one match candidate per position instead of the
  * eight-way search at the start of every token; about 3x the speed at 0.85x the ratio on text) */
 #define OTZ_M_FAST 0x100
+/* write path only: or-ed into method 8 alone (OTZ_M_DEFLATE | OTZ_M_BEST), the "best" level (libzip levels 7-9): hash
+ * chains over every position of a chunk, each position searched 128 links deep, two-step lazy parse (k_deflate_best.cuh).
+ * The chunk layout is that of the other levels.  otz_deflate_plan rejects it with OTZ_M_FAST, STORE or method 93. */
+#define OTZ_M_BEST 0x200
 
 /* One row of the device-side entry table (32 bytes). */
 typedef struct otz_entry {

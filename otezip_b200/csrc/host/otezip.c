@@ -79,7 +79,7 @@ struct otz_pending {              /* a queued source (write path) */
 	uint64_t len;
 	int owned;                    /* free(buf) after the archive is written */
 	int dirty;                    /* has bytes that zip_close must write (every new entry; a replaced existing one) */
-	int fast;                     /* zip_set_file_compression asked for level 1-3 (libzip: 1 = fastest) */
+	uint32_t level;               /* compression level asked for with zip_set_file_compression (libzip: 0 = default, 1-9) */
 	uint16_t enc;                 /* zip_file_set_encryption: AES strength 1-3, 0 = none */
 	char *pw;                     /* its password; NULL = the default password at zip_close */
 };
@@ -1529,10 +1529,12 @@ int zip_set_file_compression(zip_t *za, zip_uint64_t index, zip_int32_t comp, zi
 		return -1; /* already on disk: relabelling would corrupt it (the reference's F4 bug) */
 	}
 	za->entries[index].method = (uint16_t)comp;
-	/* comp_flags is libzip's compression level (0 = default, 1 = fastest .. 9; the reference ignores it, otezip.c:1186):
-	 * 1-3 select the compressor's single-candidate parse (OTZ_M_FAST), everything else the default eight-way search */
+	/* comp_flags is libzip's compression level (0 = default, 1 = fastest .. 9 = best; the reference ignores it,
+	 * otezip.c:1186): 1-3 select the compressor's single-candidate parse (OTZ_M_FAST), 7-9 the best level of DEFLATE
+	 * (OTZ_M_BEST: hash chains searched at every position; method 93 takes them as the default), 0 and 4-6 the
+	 * default eight-way search */
 	if (a->pend) {
-		a->pend[index].fast = comp_flags >= 1 && comp_flags <= 3;
+		a->pend[index].level = comp_flags;
 	}
 	return 0;
 }
@@ -1565,7 +1567,7 @@ int zip_file_replace(zip_t *za, zip_uint64_t index, zip_source_t *src, zip_flags
 		np.owned = 1;
 	}
 	np.dirty = 1;
-	np.fast = a->pend[index].fast; /* the level asked for with zip_set_file_compression stays with the entry */
+	np.level = a->pend[index].level; /* the level asked for with zip_set_file_compression stays with the entry */
 	np.enc = a->pend[index].enc;   /* and so does the encryption asked for with zip_file_set_encryption */
 	np.pw = a->pend[index].pw;
 	if (a->pend[index].owned) {
@@ -1862,8 +1864,11 @@ static int finalize_archive(struct otz_archive *a) {
 			/* method 93: the reference's writer cannot produce a stream its reader accepts and always falls
 			 * back to STORE (zstd.inc.c:269, otezip.c:894-899; SURVEY.md F3) — same result here */
 			method[k] = e->method == OTEZIP_METHOD_DEFLATE ? OTZ_M_DEFLATE : (e->method == OTEZIP_METHOD_ZSTD && zstd_frames ()) ? OTZ_M_ZSTD : OTZ_M_STORE;
-			if (a->pend[idx[k]].fast && method[k] != OTZ_M_STORE) {
+			const uint32_t level = a->pend[idx[k]].level;
+			if (level >= 1 && level <= 3 && method[k] != OTZ_M_STORE) {
 				method[k] |= OTZ_M_FAST;
+			} else if (level >= 7 && level <= 9 && method[k] == OTZ_M_DEFLATE) {
+				method[k] |= OTZ_M_BEST;
 			}
 			total += ((uint64_t)in_len[k] + 15) & ~15ULL;
 		}

@@ -282,6 +282,227 @@ __device__ __forceinline__ uint32_t dfl_extend(const uint32_t *__restrict__ w, u
 	return min(l, maxl);
 }
 
+// Phases 2 and 3 of a DEFLATE chunk, one warp: Huffman codes from the histograms and the extra-bit total (S.misc[0]) that
+// phase 1 left in S, the dynamic-block header, the stored-block fallback when that is not larger, and the emission of the
+// ntok tokens of tok[] (a literal is the byte, a match 0x80000000 | (dist - 1) << 8 | (len - 3)) of chunk ci = ck into
+// its output slot co; csize[ci] = bytes written.  k_deflate_chunks and k_deflate_best share it.
+__device__ __forceinline__ void dfl_code_emit(DeflateSmem &S, const uint32_t *tok, uint32_t ntok, const uint8_t *in, const OtzDflChunk &ck,
+	uint8_t *co, uint32_t *csize, uint32_t ci) {
+	const int lane = threadIdx.x & 31;
+	const uint32_t n = ck.len;
+	const uint32_t xbits = S.misc[0];
+	if (lane == 0) {
+		S.hist_ll[256] = 1;   // end of block
+	}
+	__syncwarp();
+
+	// ---------------- phase 2: Huffman codes + header cost
+	dfl_build_code(S, S.hist_ll, 286, 15, S.u.b.len_ll, S.u.b.code_ll);
+	dfl_build_code(S, S.hist_d, 30, 15, S.u.b.len_d, S.u.b.code_d);
+	// code-length sequence with zero-run RLE (symbols 17/18), then the precode
+	uint32_t hlit = 286, hdist = 30, nrle = 0;
+	if (lane == 0) {
+		while (hlit > 257 && S.u.b.len_ll[hlit - 1] == 0) {
+			hlit--;
+		}
+		while (hdist > 1 && S.u.b.len_d[hdist - 1] == 0) {
+			hdist--;
+		}
+		uint8_t *cl = S.u.b.clens;
+		for (uint32_t i = 0; i < hlit; i++) {
+			cl[i] = S.u.b.len_ll[i];
+		}
+		for (uint32_t i = 0; i < hdist; i++) {
+			cl[hlit + i] = S.u.b.len_d[i];
+		}
+		for (int i = 0; i < 19; i++) {
+			S.u.b.hist_cl[i] = 0;
+		}
+		const uint32_t tot = hlit + hdist;
+		uint8_t *rle = S.u.b.rle;   // pairs (symbol, extra value)
+		for (uint32_t i = 0; i < tot;) {
+			if (cl[i] == 0) {
+				uint32_t run = 1;
+				while (i + run < tot && cl[i + run] == 0 && run < 138) {
+					run++;
+				}
+				if (run >= 11) {
+					rle[2 * nrle] = 18;
+					rle[2 * nrle + 1] = (uint8_t)(run - 11);
+					S.u.b.hist_cl[18]++;
+					nrle++;
+					i += run;
+					continue;
+				}
+				if (run >= 3) {
+					rle[2 * nrle] = 17;
+					rle[2 * nrle + 1] = (uint8_t)(run - 3);
+					S.u.b.hist_cl[17]++;
+					nrle++;
+					i += run;
+					continue;
+				}
+			}
+			rle[2 * nrle] = cl[i];
+			rle[2 * nrle + 1] = 0;
+			S.u.b.hist_cl[cl[i]]++;
+			nrle++;
+			i++;
+		}
+	}
+	hlit = __shfl_sync(0xFFFFFFFFu, hlit, 0);
+	hdist = __shfl_sync(0xFFFFFFFFu, hdist, 0);
+	nrle = __shfl_sync(0xFFFFFFFFu, nrle, 0);
+	__syncwarp();
+	// the precode build reuses S.u.b.A/order: keep the RLE list (it lives in u.b.rle/clens)
+	dfl_build_code(S, S.u.b.hist_cl, 19, 7, S.u.b.len_cl, S.u.b.code_cl);
+	// exact size of the dynamic block
+	uint32_t bits = 0;
+	for (int s = lane; s < 286; s += 32) {
+		bits += S.hist_ll[s] * S.u.b.len_ll[s];
+	}
+	if (lane < 30) {
+		bits += S.hist_d[lane] * S.u.b.len_d[lane];
+	}
+	if (lane < 19) {
+		bits += S.u.b.hist_cl[lane] * S.u.b.len_cl[lane] + (lane == 17 ? 3 * S.u.b.hist_cl[17] : lane == 18 ? 7 * S.u.b.hist_cl[18] : 0);
+	}
+	for (int o = 16; o > 0; o >>= 1) {
+		bits += __shfl_xor_sync(0xFFFFFFFFu, bits, o);
+	}
+	bits += xbits + 3 + 14 + 19 * 3;
+	const uint32_t dyn_bytes = (bits + 3 + 7) / 8 + 4;   // + empty stored block (3 bits, pad, LEN/NLEN)
+	const uint32_t stored_bytes = 5 + n;
+	uint32_t out_bytes;
+	if (dyn_bytes >= stored_bytes) {
+		// ---------------- stored block: [BFINAL|00 padded][LEN][NLEN][bytes]
+		if (lane == 0) {
+			co[0] = (uint8_t)(ck.last & 1u);
+			co[1] = (uint8_t)(n & 0xFF);
+			co[2] = (uint8_t)(n >> 8);
+			co[3] = (uint8_t)(~n & 0xFF);
+			co[4] = (uint8_t)((~n >> 8) & 0xFF);
+		}
+		tile_copy<32>(co + 5, in + ck.in_ofs, n, lane);
+		out_bytes = stored_bytes;
+	} else {
+		// ---------------- phase 3: emit
+		DflBits bw;
+		bw.out = reinterpret_cast<uint32_t *>(co);
+		bw.acc = 0;
+		bw.nacc = 0;
+		bw.wpos = 0;
+		if (lane == 0) {
+			bw.put(0u | (2u << 1), 3);   // BFINAL=0, BTYPE=10
+			bw.put(hlit - 257, 5);
+			bw.put(hdist - 1, 5);
+			bw.put(19 - 4, 4);
+			for (int i = 0; i < 19; i++) {
+				bw.put(S.u.b.len_cl[c_cl_order[i]], 3);
+			}
+			const uint8_t *rle = S.u.b.rle;
+			for (uint32_t i = 0; i < nrle; i++) {
+				const uint32_t s = rle[2 * i];
+				bw.put(S.u.b.code_cl[s], S.u.b.len_cl[s]);
+				if (s == 17) {
+					bw.put(rle[2 * i + 1], 3);
+				} else if (s == 18) {
+					bw.put(rle[2 * i + 1], 7);
+				}
+			}
+		}
+		uint32_t wpos = __shfl_sync(0xFFFFFFFFu, bw.wpos, 0);
+		uint32_t carry = __shfl_sync(0xFFFFFFFFu, (uint32_t)bw.acc, 0);
+		uint32_t off0 = __shfl_sync(0xFFFFFFFFu, bw.nacc, 0);
+		uint32_t *out32 = reinterpret_cast<uint32_t *>(co);
+		for (uint32_t base = 0; base < ntok; base += 32) {
+			uint64_t v = 0;
+			uint32_t nb = 0;
+			if (base + lane < ntok) {
+				const uint32_t tk = tok[base + lane];
+				if (tk & 0x80000000u) {
+					uint32_t xb, xv;
+					const uint32_t ls = dfl_len_sym(tk & 0xFFu, xb, xv);
+					v = S.u.b.code_ll[ls];
+					nb = S.u.b.len_ll[ls];
+					v |= (uint64_t)xv << nb;
+					nb += xb;
+					const uint32_t ds = dfl_dist_sym((tk >> 8) & 0x7FFFu, xb, xv);
+					v |= (uint64_t)S.u.b.code_d[ds] << nb;
+					nb += S.u.b.len_d[ds];
+					v |= (uint64_t)xv << nb;
+					nb += xb;
+				} else {
+					v = S.u.b.code_ll[tk];
+					nb = S.u.b.len_ll[tk];
+				}
+			}
+			uint32_t incl = nb;
+			for (int o = 1; o < 32; o <<= 1) {
+				const uint32_t y = __shfl_up_sync(0xFFFFFFFFu, incl, o);
+				if (lane >= o) {
+					incl += y;
+				}
+			}
+			const uint32_t total = __shfl_sync(0xFFFFFFFFu, incl, 31);
+			for (int i = lane; i < 72; i += 32) {
+				S.u.b.stage[i] = (i == 0) ? carry : 0u;
+			}
+			__syncwarp();
+			if (nb) {
+				const uint32_t o = off0 + incl - nb;
+				const uint32_t wi = o >> 5, sh = o & 31u;
+				atomicOr(&S.u.b.stage[wi], (uint32_t)(v << sh));
+				const uint64_t hi = sh ? (v >> (32 - sh)) : (v >> 32);
+				if (sh + nb > 32) {
+					atomicOr(&S.u.b.stage[wi + 1], (uint32_t)hi);
+				}
+				if (sh + nb > 64) {
+					atomicOr(&S.u.b.stage[wi + 2], (uint32_t)(hi >> 32));
+				}
+			}
+			__syncwarp();
+			const uint32_t endbit = off0 + total;
+			const uint32_t nfull = endbit >> 5;
+			for (uint32_t i = lane; i < nfull; i += 32) {
+				out32[wpos + i] = S.u.b.stage[i];
+			}
+			carry = S.u.b.stage[nfull];
+			wpos += nfull;
+			off0 = endbit & 31u;
+			__syncwarp();
+		}
+		if (lane == 0) {
+			bw.wpos = wpos;
+			bw.acc = carry;
+			bw.nacc = off0;
+			bw.put(S.u.b.code_ll[256], S.u.b.len_ll[256]);   // end of block
+			bw.put(ck.last & 1u, 3);              // empty stored block: BFINAL, BTYPE=00
+			if (bw.nacc & 7) {
+				bw.put(0, 8 - (bw.nacc & 7));           // pad to a byte boundary
+			}
+			bw.put(0x0000u, 16);
+			bw.put(0xFFFFu, 16);
+			// flush the remaining whole bytes
+			uint32_t nbytes = bw.wpos * 4;
+			uint8_t *tail = co + nbytes;
+			while (bw.nacc) {
+				*tail++ = (uint8_t)bw.acc;
+				bw.acc >>= 8;
+				bw.nacc -= 8;
+				nbytes++;
+			}
+			S.misc[1] = nbytes;
+		}
+		__syncwarp();
+		out_bytes = S.misc[1];
+	}
+	if (lane == 0) {
+		csize[ci] = out_bytes;
+	}
+	__syncwarp();
+}
+
 // grid: persistent; one warp per chunk, chunks handed out in order.
 #define DFL_WARPS 3   // warps per CTA: seven CTAs (21 chunks) fit the shared memory of an SM
 // ZSTD: the job holds method-93 entries (their chunks become Zstandard blocks); a pure DEFLATE job runs the instantiation without that path
@@ -325,7 +546,7 @@ __global__ void __launch_bounds__(32 * DFL_WARPS) k_deflate_chunks(const uint8_t
 			S.misc[lane] = 0;
 		}
 		__syncwarp();
-		uint32_t ntok = 0, xbits = 0;   // tokens emitted, total extra bits (uniform)
+		uint32_t ntok = 0;   // tokens emitted (uniform)
 		uint32_t cur = 0;
 		while (cur < n) {
 			const uint32_t p = cur + lane;
@@ -479,217 +700,7 @@ __global__ void __launch_bounds__(32 * DFL_WARPS) k_deflate_chunks(const uint8_t
 			__syncwarp();
 			continue;
 		}
-		xbits = S.misc[0];
-		if (lane == 0) {
-			S.hist_ll[256] = 1;   // end of block
-		}
-		__syncwarp();
-
-		// ---------------- phase 2: Huffman codes + header cost
-		dfl_build_code(S, S.hist_ll, 286, 15, S.u.b.len_ll, S.u.b.code_ll);
-		dfl_build_code(S, S.hist_d, 30, 15, S.u.b.len_d, S.u.b.code_d);
-		// code-length sequence with zero-run RLE (symbols 17/18), then the precode
-		uint32_t hlit = 286, hdist = 30, nrle = 0;
-		if (lane == 0) {
-			while (hlit > 257 && S.u.b.len_ll[hlit - 1] == 0) {
-				hlit--;
-			}
-			while (hdist > 1 && S.u.b.len_d[hdist - 1] == 0) {
-				hdist--;
-			}
-			uint8_t *cl = S.u.b.clens;
-			for (uint32_t i = 0; i < hlit; i++) {
-				cl[i] = S.u.b.len_ll[i];
-			}
-			for (uint32_t i = 0; i < hdist; i++) {
-				cl[hlit + i] = S.u.b.len_d[i];
-			}
-			for (int i = 0; i < 19; i++) {
-				S.u.b.hist_cl[i] = 0;
-			}
-			const uint32_t tot = hlit + hdist;
-			uint8_t *rle = S.u.b.rle;   // pairs (symbol, extra value)
-			for (uint32_t i = 0; i < tot;) {
-				if (cl[i] == 0) {
-					uint32_t run = 1;
-					while (i + run < tot && cl[i + run] == 0 && run < 138) {
-						run++;
-					}
-					if (run >= 11) {
-						rle[2 * nrle] = 18;
-						rle[2 * nrle + 1] = (uint8_t)(run - 11);
-						S.u.b.hist_cl[18]++;
-						nrle++;
-						i += run;
-						continue;
-					}
-					if (run >= 3) {
-						rle[2 * nrle] = 17;
-						rle[2 * nrle + 1] = (uint8_t)(run - 3);
-						S.u.b.hist_cl[17]++;
-						nrle++;
-						i += run;
-						continue;
-					}
-				}
-				rle[2 * nrle] = cl[i];
-				rle[2 * nrle + 1] = 0;
-				S.u.b.hist_cl[cl[i]]++;
-				nrle++;
-				i++;
-			}
-		}
-		hlit = __shfl_sync(0xFFFFFFFFu, hlit, 0);
-		hdist = __shfl_sync(0xFFFFFFFFu, hdist, 0);
-		nrle = __shfl_sync(0xFFFFFFFFu, nrle, 0);
-		__syncwarp();
-		// the precode build reuses S.u.b.A/order: keep the RLE list (it lives in u.b.rle/clens)
-		dfl_build_code(S, S.u.b.hist_cl, 19, 7, S.u.b.len_cl, S.u.b.code_cl);
-		// exact size of the dynamic block
-		uint32_t bits = 0;
-		for (int s = lane; s < 286; s += 32) {
-			bits += S.hist_ll[s] * S.u.b.len_ll[s];
-		}
-		if (lane < 30) {
-			bits += S.hist_d[lane] * S.u.b.len_d[lane];
-		}
-		if (lane < 19) {
-			bits += S.u.b.hist_cl[lane] * S.u.b.len_cl[lane] + (lane == 17 ? 3 * S.u.b.hist_cl[17] : lane == 18 ? 7 * S.u.b.hist_cl[18] : 0);
-		}
-		for (int o = 16; o > 0; o >>= 1) {
-			bits += __shfl_xor_sync(0xFFFFFFFFu, bits, o);
-		}
-		bits += xbits + 3 + 14 + 19 * 3;
-		const uint32_t dyn_bytes = (bits + 3 + 7) / 8 + 4;   // + empty stored block (3 bits, pad, LEN/NLEN)
-		const uint32_t stored_bytes = 5 + n;
-		uint32_t out_bytes;
-		if (dyn_bytes >= stored_bytes) {
-			// ---------------- stored block: [BFINAL|00 padded][LEN][NLEN][bytes]
-			if (lane == 0) {
-				co[0] = (uint8_t)(ck.last & 1u);
-				co[1] = (uint8_t)(n & 0xFF);
-				co[2] = (uint8_t)(n >> 8);
-				co[3] = (uint8_t)(~n & 0xFF);
-				co[4] = (uint8_t)((~n >> 8) & 0xFF);
-			}
-			tile_copy<32>(co + 5, in + ck.in_ofs, n, lane);
-			out_bytes = stored_bytes;
-		} else {
-			// ---------------- phase 3: emit
-			DflBits bw;
-			bw.out = reinterpret_cast<uint32_t *>(co);
-			bw.acc = 0;
-			bw.nacc = 0;
-			bw.wpos = 0;
-			if (lane == 0) {
-				bw.put(0u | (2u << 1), 3);   // BFINAL=0, BTYPE=10
-				bw.put(hlit - 257, 5);
-				bw.put(hdist - 1, 5);
-				bw.put(19 - 4, 4);
-				for (int i = 0; i < 19; i++) {
-					bw.put(S.u.b.len_cl[c_cl_order[i]], 3);
-				}
-				const uint8_t *rle = S.u.b.rle;
-				for (uint32_t i = 0; i < nrle; i++) {
-					const uint32_t s = rle[2 * i];
-					bw.put(S.u.b.code_cl[s], S.u.b.len_cl[s]);
-					if (s == 17) {
-						bw.put(rle[2 * i + 1], 3);
-					} else if (s == 18) {
-						bw.put(rle[2 * i + 1], 7);
-					}
-				}
-			}
-			uint32_t wpos = __shfl_sync(0xFFFFFFFFu, bw.wpos, 0);
-			uint32_t carry = __shfl_sync(0xFFFFFFFFu, (uint32_t)bw.acc, 0);
-			uint32_t off0 = __shfl_sync(0xFFFFFFFFu, bw.nacc, 0);
-			uint32_t *out32 = reinterpret_cast<uint32_t *>(co);
-			for (uint32_t base = 0; base < ntok; base += 32) {
-				uint64_t v = 0;
-				uint32_t nb = 0;
-				if (base + lane < ntok) {
-					const uint32_t tk = tok[base + lane];
-					if (tk & 0x80000000u) {
-						uint32_t xb, xv;
-						const uint32_t ls = dfl_len_sym(tk & 0xFFu, xb, xv);
-						v = S.u.b.code_ll[ls];
-						nb = S.u.b.len_ll[ls];
-						v |= (uint64_t)xv << nb;
-						nb += xb;
-						const uint32_t ds = dfl_dist_sym((tk >> 8) & 0x7FFFu, xb, xv);
-						v |= (uint64_t)S.u.b.code_d[ds] << nb;
-						nb += S.u.b.len_d[ds];
-						v |= (uint64_t)xv << nb;
-						nb += xb;
-					} else {
-						v = S.u.b.code_ll[tk];
-						nb = S.u.b.len_ll[tk];
-					}
-				}
-				uint32_t incl = nb;
-				for (int o = 1; o < 32; o <<= 1) {
-					const uint32_t y = __shfl_up_sync(0xFFFFFFFFu, incl, o);
-					if (lane >= o) {
-						incl += y;
-					}
-				}
-				const uint32_t total = __shfl_sync(0xFFFFFFFFu, incl, 31);
-				for (int i = lane; i < 72; i += 32) {
-					S.u.b.stage[i] = (i == 0) ? carry : 0u;
-				}
-				__syncwarp();
-				if (nb) {
-					const uint32_t o = off0 + incl - nb;
-					const uint32_t wi = o >> 5, sh = o & 31u;
-					atomicOr(&S.u.b.stage[wi], (uint32_t)(v << sh));
-					const uint64_t hi = sh ? (v >> (32 - sh)) : (v >> 32);
-					if (sh + nb > 32) {
-						atomicOr(&S.u.b.stage[wi + 1], (uint32_t)hi);
-					}
-					if (sh + nb > 64) {
-						atomicOr(&S.u.b.stage[wi + 2], (uint32_t)(hi >> 32));
-					}
-				}
-				__syncwarp();
-				const uint32_t endbit = off0 + total;
-				const uint32_t nfull = endbit >> 5;
-				for (uint32_t i = lane; i < nfull; i += 32) {
-					out32[wpos + i] = S.u.b.stage[i];
-				}
-				carry = S.u.b.stage[nfull];
-				wpos += nfull;
-				off0 = endbit & 31u;
-				__syncwarp();
-			}
-			if (lane == 0) {
-				bw.wpos = wpos;
-				bw.acc = carry;
-				bw.nacc = off0;
-				bw.put(S.u.b.code_ll[256], S.u.b.len_ll[256]);   // end of block
-				bw.put(ck.last & 1u, 3);              // empty stored block: BFINAL, BTYPE=00
-				if (bw.nacc & 7) {
-					bw.put(0, 8 - (bw.nacc & 7));           // pad to a byte boundary
-				}
-				bw.put(0x0000u, 16);
-				bw.put(0xFFFFu, 16);
-				// flush the remaining whole bytes
-				uint32_t nbytes = bw.wpos * 4;
-				uint8_t *tail = co + nbytes;
-				while (bw.nacc) {
-					*tail++ = (uint8_t)bw.acc;
-					bw.acc >>= 8;
-					bw.nacc -= 8;
-					nbytes++;
-				}
-				S.misc[1] = nbytes;
-			}
-			__syncwarp();
-			out_bytes = S.misc[1];
-		}
-		if (lane == 0) {
-			csize[ci] = out_bytes;
-		}
-		__syncwarp();
+		dfl_code_emit(S, tok, ntok, in, ck, co, csize, ci);
 	}
 }
 

@@ -15,7 +15,7 @@ namespace cg = cooperative_groups;
 // -DOTZ_BOUNDS_CHECK, every OTZ_CHK site counts its violations in g_otz_violations[code], tests/test_gpu_bounds.py runs
 // the parity suite's hardest cases against that build and requires all counters to be zero (otz_debug_violations).
 // In the release build the macro compiles to nothing.
-#define OTZ_CHK_SLOTS 24
+#define OTZ_CHK_SLOTS 27
 #ifdef OTZ_BOUNDS_CHECK
 __device__ unsigned long long g_otz_violations[OTZ_CHK_SLOTS];
 #define OTZ_CHK(cond, code)                                     \
@@ -51,6 +51,9 @@ __device__ unsigned long long g_otz_violations[OTZ_CHK_SLOTS];
 #define OTZ_CK_AES_IN 21        // k_aes_ctr: load outside the input buffer
 #define OTZ_CK_D64_OUT 22       // k_inflate<D64>: piece of a long match beyond the entry's output slice
 #define OTZ_CK_D64_SRC 23       // k_inflate<D64>: piece source neither in the ring nor flushed to HBM, or before the slice
+#define OTZ_CK_DFB_LINK 24      // k_deflate_best: hash-chain link that is not an earlier position of the chunk
+#define OTZ_CK_DFB_STAGE 25     // k_deflate_best: word read beyond the staged chunk
+#define OTZ_CK_DFB_STORE 26     // k_deflate_best: match-table / token store outside the slot, or ahead of the parse
 
 #define OTZ_SIG_LFH 0x04034b50u
 #define OTZ_MAX_PAYLOAD (2ull * 1024ull * 1024ull * 1024ull)  // otezip.c:102

@@ -15,6 +15,7 @@
 #include "k_inflate2.cuh"
 #include "k_inflate3.cuh"
 #include "k_deflate.cuh"
+#include "k_deflate_best.cuh"
 #include "k_resolve.cuh"
 #include "k_zstd_tok.cuh"
 #include "k_aes.cuh"
@@ -1733,6 +1734,8 @@ extern "C" int otz_status_accepts(int32_t st, int verify_crc, int ref_compat) {
 struct otz_deflate_job {
 	bool has_zstd;   // some entry asks for method 93: the compressor instantiation with the Zstandard block writer
 	uint32_t n, n_chunks, n_crc_chunks, n_slots;
+	uint32_t n_def_chunks;   // chunks [0, n_def_chunks) run on k_deflate_chunks, the best-level chunks behind them on k_deflate_best
+	int best_grid;
 	uint64_t in_total;
 	OtzDflEntry *d_ents;
 	OtzDflChunk *d_chunks;
@@ -1786,20 +1789,31 @@ extern "C" int otz_deflate_plan(otz_ctx *c, const uint64_t *in_ofs, const uint32
 	std::vector<otz_entry> cents(n);
 	std::vector<OtzCrcChunk> cchunks;
 	uint64_t total = 0;
+	std::vector<OtzDflChunk> bchunks;   // best-level chunks, placed behind all others
+	std::vector<uint8_t> is_best(n);
 	for (uint32_t i = 0; i < n; i++) {
-		const uint16_t m_i = method[i] & (uint16_t)~OTZ_M_FAST;
+		const uint16_t m_i = method[i] & (uint16_t)~(OTZ_M_FAST | OTZ_M_BEST);
 		const uint32_t fast_i = (method[i] & OTZ_M_FAST) ? 8u : 0u;
+		const bool best_i = (method[i] & OTZ_M_BEST) != 0;
 		if (m_i != OTZ_M_STORE && m_i != OTZ_M_DEFLATE && m_i != OTZ_M_ZSTD) {
 			delete j;
 			snprintf(g_err, sizeof(g_err), "otz_deflate_plan: method %u is not on the GPU write path", method[i]);
 			return OTZ_ERR_ARG;
 		}
+		if (best_i && (fast_i || m_i != OTZ_M_DEFLATE)) {
+			delete j;
+			snprintf(g_err, sizeof(g_err), "otz_deflate_plan: method 0x%x: OTZ_M_BEST is a level of DEFLATE (8) only and excludes OTZ_M_FAST",
+				method[i]);
+			return OTZ_ERR_ARG;
+		}
+		std::vector<OtzDflChunk> &cv = best_i ? bchunks : chunks;
 		OtzDflEntry &e = ents[i];
 		e.in_ofs = in_ofs[i];
 		e.len = in_len[i];
 		e.method_in = m_i;
 		e.pad = 0;
-		e.first_chunk = (uint32_t)chunks.size();
+		is_best[i] = best_i;   // (first_chunk counts within bchunks until the two lists are joined)
+		e.first_chunk = (uint32_t)cv.size();
 		const uint32_t nc = (in_len[i] + DFL_CHUNK - 1) / DFL_CHUNK;
 		e.n_chunks = nc;
 		for (uint32_t k = 0; k < nc; k++) {
@@ -1810,7 +1824,7 @@ extern "C" int otz_deflate_plan(otz_ctx *c, const uint64_t *in_ofs, const uint32
 			ck.last = (k + 1 == nc ? 1u : 0u) | (k == 0 ? 2u : 0u) | (m_i == OTZ_M_ZSTD ? 4u : 0u) | fast_i;
 			ck.pad = in_len[i];
 			j->has_zstd = j->has_zstd || m_i == OTZ_M_ZSTD;
-			chunks.push_back(ck);
+			cv.push_back(ck);
 		}
 		otz_entry &ce = cents[i];
 		memset(&ce, 0, sizeof(ce));
@@ -1823,12 +1837,34 @@ extern "C" int otz_deflate_plan(otz_ctx *c, const uint64_t *in_ofs, const uint32
 		}
 		total += in_len[i];
 	}
+	j->n_def_chunks = (uint32_t)chunks.size();
+	for (uint32_t i = 0; i < n; i++) {
+		if (is_best[i]) {
+			ents[i].first_chunk += j->n_def_chunks;
+		}
+	}
+	chunks.insert(chunks.end(), bchunks.begin(), bchunks.end());
 	j->n_chunks = (uint32_t)chunks.size();
 	j->n_crc_chunks = (uint32_t)cchunks.size();
 	j->in_total = total;
 	// persistent grid for the compressor: 2 CTAs x 8 warps per SM
-	j->grid = std::max(1, std::min<int>(c->sm_count * 7, (int)((j->n_chunks + DFL_WARPS - 1) / DFL_WARPS)));
+	j->grid = std::max(1, std::min<int>(c->sm_count * 7, (int)((j->n_def_chunks + DFL_WARPS - 1) / DFL_WARPS)));
 	j->n_slots = (uint32_t)j->grid * DFL_WARPS;
+	// best level: one CTA per chunk, as many as fit the device; the CTAs use token slots of their own, shared with the
+	// default kernel, which runs before them on the same stream
+	const uint32_t n_best = j->n_chunks - j->n_def_chunks;
+	if (n_best) {
+		int per_sm = 0;
+		CK(cudaFuncSetAttribute(k_deflate_best, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)DFB_SMEM));
+		CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_deflate_best, DFB_THREADS, DFB_SMEM));
+		if (per_sm < 1) {
+			otz_deflate_destroy(c, j);
+			snprintf(g_err, sizeof(g_err), "otz_deflate_plan: k_deflate_best does not fit an SM");
+			return OTZ_ERR_CUDA;
+		}
+		j->best_grid = (int)std::min<uint32_t>((uint32_t)(c->sm_count * per_sm), n_best);
+	}
+	const size_t tok_slots = std::max<size_t>(j->n_slots, (size_t)j->best_grid);
 	int rc;
 	if ((rc = upload(&j->d_ents, ents, c->stream)) || (rc = upload(&j->d_chunks, chunks, c->stream)) ||
 		(rc = upload(&j->d_crc_ents, cents, c->stream)) || (rc = upload(&j->d_crc_chunks, cchunks, c->stream))) {
@@ -1838,7 +1874,7 @@ extern "C" int otz_deflate_plan(otz_ctx *c, const uint64_t *in_ofs, const uint32
 	const size_t n1 = std::max<uint32_t>(n, 1), nc1 = std::max<uint32_t>(j->n_chunks, 1);
 	bool ok = cudaMalloc(&j->d_est, n1 * sizeof(OtzEntryState)) == cudaSuccess && cudaMalloc(&j->d_status, n1 * 4) == cudaSuccess &&
 		cudaMalloc(&j->d_acc, n1 * 4) == cudaSuccess && cudaMalloc(&j->d_crc, n1 * 4) == cudaSuccess &&
-		cudaMalloc(&j->d_tokens, (size_t)j->n_slots * DFL_CHUNK * 4) == cudaSuccess &&
+		cudaMalloc(&j->d_tokens, tok_slots * DFL_CHUNK * 4) == cudaSuccess &&
 		cudaMalloc(&j->d_cout, nc1 * (size_t)DFL_OUT_STRIDE) == cudaSuccess && cudaMalloc(&j->d_csize, nc1 * 4) == cudaSuccess &&
 		cudaMalloc(&j->d_out_size, n1 * 4) == cudaSuccess && cudaMalloc(&j->d_method_out, n1 * 2) == cudaSuccess &&
 		cudaMalloc(&j->d_out_ofs, n1 * 8) == cudaSuccess && cudaMalloc(&j->d_total, 8) == cudaSuccess &&
@@ -1877,7 +1913,7 @@ extern "C" int otz_deflate_run(otz_ctx *c, otz_deflate_job *j, const uint8_t *d_
 	}
 	k_crc_finalize<<<(n + 255) / 256, 256, 0, s>>>(j->d_crc_ents, n, j->d_acc, j->d_crc, j->d_status, c->d_tabs);
 	c->launches++;
-	if (j->n_chunks) {
+	if (j->n_def_chunks) {
 		const size_t smem = DFL_WARPS * sizeof(DeflateSmem);
 		static bool attr_done = false;
 		if (!attr_done) {
@@ -1886,7 +1922,12 @@ extern "C" int otz_deflate_run(otz_ctx *c, otz_deflate_job *j, const uint8_t *d_
 			attr_done = true;
 		}
 		auto kern = j->has_zstd ? k_deflate_chunks<true> : k_deflate_chunks<false>;
-		kern<<<j->grid, 32 * DFL_WARPS, smem, s>>>(d_in, j->d_chunks, j->n_chunks, j->d_tokens, j->d_cout, j->d_csize, j->d_counter, j->n_slots);
+		kern<<<j->grid, 32 * DFL_WARPS, smem, s>>>(d_in, j->d_chunks, j->n_def_chunks, j->d_tokens, j->d_cout, j->d_csize, j->d_counter, j->n_slots);
+		c->launches++;
+	}
+	if (j->best_grid) {
+		k_deflate_best<<<j->best_grid, DFB_THREADS, DFB_SMEM, s>>>(d_in, j->d_chunks, j->n_def_chunks, j->n_chunks - j->n_def_chunks, j->d_tokens,
+			j->d_cout, j->d_csize, j->d_counter + 1);
 		c->launches++;
 	}
 	k_deflate_entry_sizes<<<(n + 255) / 256, 256, 0, s>>>(j->d_ents, n, j->d_csize, j->d_out_size, j->d_method_out);

@@ -4,7 +4,7 @@
 // is the entropy of the token histograms + extra bits + a header guess (within 1 % of what the GPU encoder produces).
 //   gcc -O2 -o dfl_parse_sim tools/dfl_parse_sim.c -lm
 //   ./dfl_parse_sim corpus.bin [hb=<hash bits>] [ways=<bucket ways>] [one] [lazy2=1] [twopass=1] [first4] [insall] [rep]
-//                   [chain=<depth>] [adapt=<pairs>] [nice=<len>]
+//                   [chain=<depth>] [adapt=<pairs>] [nice=<len>] [best [minm=3|4]]
 //   (corpus.bin: 32 x 256 KiB slices of synth.TextPool(seed=5), the corpus of bench.py --workload c5)
 // Results that shaped the kernel (ratio on that corpus; zlib level 6: 9.38):
 //   hb=12 ways=1 one                      6.85   round 1 (measured on the GPU: 6.87)
@@ -15,7 +15,17 @@
 //   hb=9 ways=8 one lazy2=1 twopass=1     8.23   searched at the token starts of a first pass -> default level (GPU: 8.25 at 29.8 GB/s)
 //   hb=9 ways=8 one lazy2=1 twopass=1 adapt=32   8.00   at most 32 (token, way) pairs per step
 //   hb=9 ways=8 one lazy2=1 first4        7.05   first way whose four bytes match, no second pass
-//   hb=8 ways=16 one / hb=15 chain=16     8.37 / 9.01
+//   hb=8 ways=16 one / hb=15 chain=16     8.37 / 8.92   (chain=: the ways, then the chain behind the oldest one, to <depth> links)
+// Best level (`best`: exact chains over all positions, every position searched on its own, zlib's lazy parse; zlib-6 on
+// whole entries 9.38, zlib-9 on independent 65,280-byte chunks 9.69):
+//   best hb=15 minm=4 chain=4096 nice=258            9.71   zlib's level-9 search, one-step lazy rule
+//   best hb=15 minm=3 chain=4096 nice=258            9.65   minimum match 3 (with TOO_FAR) loses in one Huffman block
+//   best hb=15 minm=4 chain=128 nice=128             9.62
+//   best hb=14 minm=4 lazy2=1 nice=258 chain=8 / 16 / 32 / 64   8.94 / 9.29 / 9.54 / 9.74   two-step lazy rule
+//   best hb=14 minm=4 lazy2=1 nice=258 chain=128     9.91   -> best level (k_deflate_best.cuh)
+//   best hb=14 minm=4 lazy2=1 nice=258 chain=256 / 4096   10.00 / 10.01
+//   best hb=14 minm=3 lazy2=1 chain=32 9.33; hb=13 = hb=14; nice=128 = nice=258 at chain=64
+// A cost-based parse was not modelled: the lazy rule clears the bar with 5 % to spare.
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
@@ -49,6 +59,7 @@ static double chunk_bits(const uint8_t*d,uint32_t n){
       int wmax = TWOPASS ? 1 : WAYS;
       if(FIRST4){ for(int w=0;w<WAYS;w++){uint32_t c=cand[l][w]; if(c&&p-(c-1)<=32768&&rd32(d+c-1)==rd32(d+p)){int L=mlen_at(d,n,p,c-1); if(L>=MINM){mlen[l]=L;mdist[l]=p-(c-1);} break;}} continue; }
       for(int w=0;w<wmax;w++){uint32_t c=cand[l][w]; if(c&&p-(c-1)<=32768){int L=mlen_at(d,n,p,c-1); if(L>=MINM&&L>(int)mlen[l]){mlen[l]=L;mdist[l]=p-(c-1);}}}
+      if(CHAIN){uint32_t c=cand[l][WAYS-1]; for(int k=0;k<CHAIN&&c;k++){c=prev[c-1]; if(!c||p-(c-1)>32768)break; int L=mlen_at(d,n,p,c-1); if(L>=MINM&&L>(int)mlen[l]){mlen[l]=L;mdist[l]=p-(c-1);}}}
     }
     if(TWOPASS){ for(int pass=0;pass<TWOPASS;pass++){ uint32_t i=0; uint32_t lim=n-cur<32?n-cur:32; int start[32]={0};
         while(i<lim){uint32_t L=mlen[i],Ln=(i+1<32)?mlen[i+1]:0; uint32_t Ln2=(i+2<32)?mlen[i+2]:0; start[i]=1; if(L>=MINM&&Ln<=L&&!(LAZY2&&Ln2>L+1)) i+=L; else i++;}
@@ -67,7 +78,25 @@ static double chunk_bits(const uint8_t*d,uint32_t n){
   hl[256]=1; double tl=0,td=0,bits=0; for(int i=0;i<286;i++)tl+=hl[i]; for(int i=0;i<30;i++)td+=hd[i];
   for(int i=0;i<286;i++)if(hl[i])bits+=-hl[i]*log2(hl[i]/tl); for(int i=0;i<30;i++)if(hd[i])bits+=-hd[i]*log2(hd[i]/td);
   free(ht); if(prev)free(prev); return bits*1.005+xbits+ 90*8 + 5*8; }
-int main(int argc,char**argv){ for(int i=2;i<argc;i++){ if(!strncmp(argv[i],"hb=",3))HB=atoi(argv[i]+3); if(!strcmp(argv[i],"insall"))INSALL=1; if(!strcmp(argv[i],"rep"))REP=1; if(!strncmp(argv[i],"ways=",5))WAYS=atoi(argv[i]+5); if(!strncmp(argv[i],"chain=",6))CHAIN=atoi(argv[i]+6); if(!strcmp(argv[i],"one"))ONE=1; if(!strcmp(argv[i],"first4"))FIRST4=1; if(!strncmp(argv[i],"adapt=",6))ADAPT=atoi(argv[i]+6); if(!strncmp(argv[i],"nice=",5))NICE=atoi(argv[i]+5); if(!strncmp(argv[i],"twopass=",8))TWOPASS=atoi(argv[i]+8); if(!strncmp(argv[i],"lazy2=",6))LAZY2=atoi(argv[i]+6);}
+// BEST: the scheme of k_deflate_best (k_deflate_best.cuh).  Hash chains over every position of the chunk (hash of the first
+// MINB bytes, HB bits; chains are exact: the warp-serial insertion of the kernel links equal-hash lanes in position order),
+// every position searched on its own to CHAIN links with an early exit at NICE (longest wins, the nearer on equal lengths),
+// then zlib's lazy parse over the per-position matches (a match is taken unless the next position has a longer one;
+// lazy2=1 also looks two ahead), a length-3 match farther than 4,096 bytes is dropped (zlib's TOO_FAR).
+static int BEST=0, MINB=4;
+static double chunk_bits_best(const uint8_t*d,uint32_t n){
+  uint32_t hs=1u<<HB; uint16_t*head=calloc(hs,2); uint16_t*prev=calloc(CHUNK,2); uint16_t*ml=calloc(n+2,2); uint16_t*md=calloc(n+2,2);
+  double hl[286]={0},hd[30]={0}; double xbits=0;
+  for(uint32_t p=0;p+MINB<=n;p++){uint32_t v=rd32(d+p); if(MINB==3)v&=0xFFFFFF; uint32_t h=(v*2654435761u)>>(32-HB); prev[p]=head[h]; head[h]=p+1;
+    uint32_t best=0,bd=0,maxl=n-p<MAXM?n-p:MAXM; uint32_t c=prev[p];
+    for(int k=0;k<CHAIN&&c;k++,c=prev[c-1]){ if(p-(c-1)>32768)break; if(d[c-1+best]!=d[p+best])continue; uint32_t L=mlen_at(d,n,p,c-1); if(L>best){best=L;bd=p-(c-1); if(L>=(uint32_t)NICE||L==maxl)break;}}
+    if(best>=(uint32_t)MINB&&!(best==3&&bd>4096)){ml[p]=best;md[p]=bd;} }
+  uint32_t i=0; while(i<n){uint32_t L=ml[i]; uint32_t Ln=i+1<n?ml[i+1]:0, Ln2=i+2<n?ml[i+2]:0;
+    if(L&&Ln<=L&&!(LAZY2&&Ln2>L+1)){int s=lsym(L);hl[257+s]++;xbits+=lext[s];int ds=dsym(md[i]);hd[ds]++;xbits+=dext[ds];i+=L;} else {hl[d[i]]++;i++;}}
+  hl[256]=1; double tl=0,td=0,bits=0; for(int k=0;k<286;k++)tl+=hl[k]; for(int k=0;k<30;k++)td+=hd[k];
+  for(int k=0;k<286;k++)if(hl[k])bits+=-hl[k]*log2(hl[k]/tl); for(int k=0;k<30;k++)if(hd[k])bits+=-hd[k]*log2(hd[k]/td);
+  free(head);free(prev);free(ml);free(md); return bits*1.005+xbits+ 90*8 + 5*8; }
+int main(int argc,char**argv){ for(int i=2;i<argc;i++){ if(!strncmp(argv[i],"hb=",3))HB=atoi(argv[i]+3); if(!strcmp(argv[i],"insall"))INSALL=1; if(!strcmp(argv[i],"rep"))REP=1; if(!strncmp(argv[i],"ways=",5))WAYS=atoi(argv[i]+5); if(!strncmp(argv[i],"chain=",6))CHAIN=atoi(argv[i]+6); if(!strcmp(argv[i],"one"))ONE=1; if(!strcmp(argv[i],"best"))BEST=1; if(!strncmp(argv[i],"minm=",5))MINB=atoi(argv[i]+5); if(!strcmp(argv[i],"first4"))FIRST4=1; if(!strncmp(argv[i],"adapt=",6))ADAPT=atoi(argv[i]+6); if(!strncmp(argv[i],"nice=",5))NICE=atoi(argv[i]+5); if(!strncmp(argv[i],"twopass=",8))TWOPASS=atoi(argv[i]+8); if(!strncmp(argv[i],"lazy2=",6))LAZY2=atoi(argv[i]+6);}
   FILE*f=fopen(argv[1],"rb"); fseek(f,0,SEEK_END); long sz=ftell(f); fseek(f,0,SEEK_SET); uint8_t*d=malloc(sz+16); fread(d,1,sz,f); memset(d+sz,0,16);
-  double bits=0; for(long e=0;e<sz;e+=262144){long en=sz-e<262144?sz-e:262144; for(long o=0;o<en;o+=CHUNK){uint32_t n=en-o<CHUNK?en-o:CHUNK; bits+=chunk_bits(d+e+o,n);}}
+  double bits=0; for(long e=0;e<sz;e+=262144){long en=sz-e<262144?sz-e:262144; for(long o=0;o<en;o+=CHUNK){uint32_t n=en-o<CHUNK?en-o:CHUNK; bits+=BEST?chunk_bits_best(d+e+o,n):chunk_bits(d+e+o,n);}}
   printf("nice=%d pairs/step %.1f ",NICE,nsteps?(double)npairs_tot/nsteps:0.0); printf("HB=%d ways=%d chain=%d insall=%d rep=%d one=%d ratio %.3f\n",HB,WAYS,CHAIN,INSALL,REP,ONE,sz*8.0/bits); }
