@@ -1,7 +1,7 @@
 /* otezip/config.h — build switches and method ids of the B200 build.
  * Same macro names and values as the reference's src/include/otezip/config.h:6-35 (the method ids are
- * the ZIP APPNOTE numbers and part of the on-disk format); only methods 0, 8 and 93 are implemented
- * by the GPU path, the rest are reported as unsupported (OTZ_ST_METHOD). */
+ * the ZIP APPNOTE numbers and part of the on-disk format); methods 0, 8 and 93 are implemented by the GPU path, which also
+ * reads 9 (Deflate64) and 95 (XZ, otz_gpu.h: OTZ_M_XZ); the rest are reported as unsupported (OTZ_ST_METHOD). */
 #ifndef OTEZIP_CONFIG_H
 #define OTEZIP_CONFIG_H
 

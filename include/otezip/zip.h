@@ -104,6 +104,11 @@ typedef struct zip_source otezip_src_buf;
  * reference rejects the method, so with the default otezip_ref_compat = 1 zip_fopen_index returns NULL for such an entry
  * (otezip_b200_entry_status: OTZ_ST_OK | OTZ_STF_REF_EOB when its stream is valid); with 0 it hands out the bytes. */
 #define ZIP_CM_DEFLATE64 9
+/* XZ (xz streams with one LZMA2 filter; libzip ZIP_CM_XZ, 7-Zip -mm=xz): read only, under the same rule as Deflate64 --
+ * with otezip_ref_compat = 1 zip_fopen_index returns NULL for such an entry (otezip_b200_entry_status: OTZ_ST_OK |
+ * OTZ_STF_REF_EOB when its payload is valid); with 0 it hands out the bytes.  Filters other than LZMA2 (BCJ, delta) give
+ * OTZ_ST_METHOD. */
+#define ZIP_CM_XZ 95
 
 #define ZIP_UINT64_MAX ((zip_uint64_t)-1)
 
@@ -197,7 +202,7 @@ int zip_set_default_password(zip_t *za, const char *password);   /* NULL clears 
 zip_file_t *zip_fopen_index_encrypted(zip_t *za, zip_uint64_t index, zip_flags_t flags, const char *password);
 int zip_file_set_encryption(zip_t *za, zip_uint64_t index, zip_uint16_t method, const char *password);   /* NULL: the default */
 int zip_encryption_method_supported(zip_uint16_t method, int encode);
-/* libzip: 1 when entries of this compression method can be read (compress == 0: 0, 8, 9, 93) or written (compress != 0:
+/* libzip: 1 when entries of this compression method can be read (compress == 0: 0, 8, 9, 93, 95) or written (compress != 0:
  * 0, 8, 93) */
 int zip_compression_method_supported(zip_int32_t method, int compress);
 
@@ -218,7 +223,7 @@ extern uint64_t otezip_max_expansion_ratio;   /* zip-bomb guard: uncomp <= comp*
 extern uint64_t otezip_max_expansion_slack;
 extern int otezip_ignore_zipbomb;
 /* B200 build: 1 (default) reproduces the reference inflater's end-of-input rule (SURVEY.md F1) so that
- * accept/reject is bit-identical; 0 accepts every valid RFC 1951 stream, and Deflate64 entries.  The environment variable
+ * accept/reject is bit-identical; 0 accepts every valid RFC 1951 stream, and Deflate64 and XZ entries.  The environment variable
  * OTEZIP_REF_COMPAT=0 sets the initial value (read when the library is loaded). */
 extern int otezip_ref_compat;
 /* Extension (SURVEY.md §8f rank 2): 1 = zip_close writes every entry in the STREAMING layout — general-purpose flag

@@ -50,7 +50,7 @@ extern "C" {
 #define OTZ_ST_LFH_SIG 2       /* LFH signature mismatch                          otezip.c:421-423 */
 #define OTZ_ST_DATA_RANGE 3    /* payload outside the image                       otezip.c:438-446 */
 #define OTZ_ST_ZIPBOMB 4       /* uncomp > comp*ratio+slack                       otezip.c:454-462 */
-#define OTZ_ST_METHOD 5        /* method not on the GPU path (only 0, 8, 9, 93)   otezip.c:662-665 */
+#define OTZ_ST_METHOD 5        /* method not on the GPU path (only 0, 8, 9, 93, 95; XZ: a filter other than LZMA2) otezip.c:662-665 */
 #define OTZ_ST_STORE_SIZE 6    /* STORE with comp != uncomp                       otezip.c:482-485 */
 #define OTZ_ST_DATA 7          /* corrupt stream (Z_DATA_ERROR class)             dec / zstd */
 #define OTZ_ST_TRUNCATED 8     /* input exhausted before the stream ended (Z_BUF_ERROR class) */
@@ -73,6 +73,9 @@ extern "C" {
  * method, so a stream that decodes carries OTZ_STF_REF_EOB as well (handed out only when ref_compat is 0). */
 #define OTZ_M_DEFLATE64 9
 #define OTZ_M_ZSTD 93
+/* read path only: XZ (xz streams of one LZMA2 filter each), walked by k_xz_walk and decoded by k_lzma.  The reference rejects
+ * the method, so a payload that decodes carries OTZ_STF_REF_EOB as well (handed out only when ref_compat is 0). */
+#define OTZ_M_XZ 95
 /* write path only: or-ed into method[i], compression level 1 ("fastest": one match candidate per position instead of the
  * eight-way search at the start of every token; about 3x the speed at 0.85x the ratio on text) */
 #define OTZ_M_FAST 0x100

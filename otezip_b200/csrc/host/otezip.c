@@ -50,7 +50,7 @@ int otezip_write_data_descriptors = 0;
 int otezip_zstd_frames = 0;
 
 /* OTEZIP_REF_COMPAT=0 in the environment sets the initial value of otezip_ref_compat, so that a program that never touches
- * the global (the otezip CLI) can extract what the reference rejects: Deflate64 entries, F1 streams, real Zstandard frames.
+ * the global (the otezip CLI) can extract what the reference rejects: Deflate64 and XZ entries, F1 streams, real Zstandard frames.
  * Read once, when the library is loaded; a program that assigns the global later still wins. */
 __attribute__ ((constructor)) static void otezip_env_defaults(void) {
 	const char *e = getenv ("OTEZIP_REF_COMPAT");
@@ -411,7 +411,8 @@ static int load_central(struct otz_archive *a) {
 					const uint8_t *d = x + xo + 4;
 					const uint16_t ver = sz == 7 ? otezip_read_le16 (d) : 0, am = sz == 7 ? otezip_read_le16 (d + 5) : 0xFFFF;
 					if ((ver == 1 || ver == 2) && d[2] == 'A' && d[3] == 'E' && d[4] >= 1 && d[4] <= 3 &&
-						(am == OTEZIP_METHOD_STORE || am == OTEZIP_METHOD_DEFLATE || am == OTZ_M_DEFLATE64 || am == OTEZIP_METHOD_ZSTD)) {
+						(am == OTEZIP_METHOD_STORE || am == OTEZIP_METHOD_DEFLATE || am == OTZ_M_DEFLATE64 || am == OTEZIP_METHOD_ZSTD ||
+						 am == OTZ_M_XZ)) {
 						a->aes[i].vendor = ver;
 						a->aes[i].strength = d[4];
 						a->aes[i].method = am;
@@ -858,7 +859,7 @@ static int32_t host_precheck(const struct otz_archive *a, zip_uint64_t i, const 
 		if (inner_comp (a, i) != e->uncomp_size) {
 			return OTZ_ST_STORE_SIZE;
 		}
-	} else if (method != OTEZIP_METHOD_DEFLATE && method != OTZ_M_DEFLATE64 && method != OTEZIP_METHOD_ZSTD) {
+	} else if (method != OTEZIP_METHOD_DEFLATE && method != OTZ_M_DEFLATE64 && method != OTEZIP_METHOD_ZSTD && method != OTZ_M_XZ) {
 		return OTZ_ST_METHOD;
 	}
 	if (x && !pw) {
@@ -1356,7 +1357,7 @@ int zip_compression_method_supported(zip_int32_t method, int compress) {
 	if (method == ZIP_CM_STORE || method == ZIP_CM_DEFLATE || method == OTEZIP_METHOD_ZSTD) {
 		return 1;
 	}
-	return !compress && method == ZIP_CM_DEFLATE64;   /* Deflate64 is read, never written */
+	return !compress && (method == ZIP_CM_DEFLATE64 || method == ZIP_CM_XZ);   /* Deflate64 and XZ are read, never written */
 }
 
 int zip_encryption_method_supported(zip_uint16_t method, int encode) {

@@ -61,7 +61,7 @@ __global__ void k_resolve(const uint8_t *__restrict__ archive, uint64_t archive_
 				st = OTZ_ST_STORE_SIZE;
 				break;
 			}
-		} else if (e.method != OTZ_M_DEFLATE && e.method != OTZ_M_DEFLATE64 && e.method != OTZ_M_ZSTD) {  // otezip.c:662-665
+		} else if (e.method != OTZ_M_DEFLATE && e.method != OTZ_M_DEFLATE64 && e.method != OTZ_M_ZSTD && e.method != OTZ_M_XZ) {  // otezip.c:662-665
 			st = OTZ_ST_METHOD;
 			break;
 		}

@@ -15,7 +15,7 @@ namespace cg = cooperative_groups;
 // -DOTZ_BOUNDS_CHECK, every OTZ_CHK site counts its violations in g_otz_violations[code], tests/test_gpu_bounds.py runs
 // the parity suite's hardest cases against that build and requires all counters to be zero (otz_debug_violations).
 // In the release build the macro compiles to nothing.
-#define OTZ_CHK_SLOTS 27
+#define OTZ_CHK_SLOTS 31
 #ifdef OTZ_BOUNDS_CHECK
 __device__ unsigned long long g_otz_violations[OTZ_CHK_SLOTS];
 #define OTZ_CHK(cond, code)                                     \
@@ -54,6 +54,10 @@ __device__ unsigned long long g_otz_violations[OTZ_CHK_SLOTS];
 #define OTZ_CK_DFB_LINK 24      // k_deflate_best: hash-chain link that is not an earlier position of the chunk
 #define OTZ_CK_DFB_STAGE 25     // k_deflate_best: word read beyond the staged chunk
 #define OTZ_CK_DFB_STORE 26     // k_deflate_best: match-table / token store outside the slot, or ahead of the parse
+#define OTZ_CK_XZ_SEG 27        // k_xz_walk: segment beyond the entry's slot range of the segment table
+#define OTZ_CK_XZ_IN 28         // k_lzma: uncompressed-chunk load beyond the entry's payload
+#define OTZ_CK_XZ_PROB 29       // k_lzma: probability index beyond the model of the segment's class
+#define OTZ_CK_XZ_OUT 30        // k_lzma: output store beyond the segment's part of the entry's slice
 
 #define OTZ_SIG_LFH 0x04034b50u
 #define OTZ_MAX_PAYLOAD (2ull * 1024ull * 1024ull * 1024ull)  // otezip.c:102

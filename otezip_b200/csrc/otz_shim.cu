@@ -19,6 +19,7 @@
 #include "k_resolve.cuh"
 #include "k_zstd_tok.cuh"
 #include "k_aes.cuh"
+#include "k_xz.cuh"
 #include "otz_common.cuh"
 
 static thread_local char g_err[512] = "";
@@ -80,6 +81,8 @@ struct otz_ctx {
 	struct OtzAesRun *aes;  // device state of the last otz_aes_open / otz_aes_seal (created on first use)
 	cudaStream_t stream_d64[2];   // Deflate64 entries (large / small), beside the DEFLATE work of the same run
 	cudaEvent_t ev_d64_fork, ev_d64_join[2];
+	cudaStream_t stream_xz;       // XZ entries: walk, decode, verdicts, beside the other work of the same run
+	cudaEvent_t ev_xz_fork, ev_xz_join;
 };
 
 struct otz_plan {
@@ -108,6 +111,10 @@ struct otz_plan {
 	uint32_t n_zchunks;
 	uint32_t *d_d64_list, n_d64;   // Deflate64 entries (method 9), longest first; [0, n_d64_big) are the large ones
 	uint32_t n_d64_big;
+	uint32_t *d_xz_list, n_xz;     // XZ entries (method 95), longest first
+	XzEnt *d_xz_ent;               // per list slot: its range of the segment table, the walk's and the segments' verdicts
+	XzSeg *d_xz_segs;              // segment table: floor(uncomp_size / XZ_SEG_MIN) + 1 slots per entry, in list order
+	uint32_t n_xz_slots;
 	uint64_t *d_ztok_ofs;      // two-phase Zstandard: token scratch offset of every method-93 list slot (+ end)
 	uint64_t ztok_bytes;
 	I2TokRes *d_ztokres;
@@ -231,6 +238,9 @@ extern "C" int otz_ctx_create(int device, otz_ctx **out) {
 		CK(cudaEventCreateWithFlags(&c->ev_d64_join[k], cudaEventDisableTiming));
 	}
 	CK(cudaEventCreateWithFlags(&c->ev_d64_fork, cudaEventDisableTiming));
+	CK(cudaStreamCreateWithFlags(&c->stream_xz, cudaStreamNonBlocking));
+	CK(cudaEventCreateWithFlags(&c->ev_xz_fork, cudaEventDisableTiming));
+	CK(cudaEventCreateWithFlags(&c->ev_xz_join, cudaEventDisableTiming));
 	CK(cudaEventCreate(&c->ev0));
 	CK(cudaEventCreate(&c->ev1));
 	for (auto &slot : c->pev) {
@@ -304,6 +314,9 @@ extern "C" void otz_ctx_destroy(otz_ctx *c) {
 	cudaEventDestroy(c->ev_join3);
 	cudaEventDestroy(c->ev_join4);
 	cudaEventDestroy(c->ev_d64_fork);
+	cudaEventDestroy(c->ev_xz_fork);
+	cudaEventDestroy(c->ev_xz_join);
+	cudaStreamDestroy(c->stream_xz);
 	for (int k = 0; k < 2; k++) {
 		cudaEventDestroy(c->ev_d64_join[k]);
 		cudaStreamDestroy(c->stream_d64[k]);
@@ -473,6 +486,9 @@ extern "C" void otz_plan_destroy(otz_ctx *c, otz_plan *p) {
 	cudaFree(p->d_zstd_list);
 	cudaFree(p->d_zchunks);
 	cudaFree(p->d_d64_list);
+	cudaFree(p->d_xz_list);
+	cudaFree(p->d_xz_ent);
+	cudaFree(p->d_xz_segs);
 	cudaFree(p->d_ztok_ofs);
 	cudaFree(p->d_ztokres);
 	cudaFree(p->d_counter);
@@ -502,7 +518,7 @@ extern "C" int otz_plan_create(otz_ctx *c, const otz_entry *ents, uint32_t n, co
 	}
 	// Work lists.  CRC chunks: STORE entries first (they are also the copy list), then the rest.
 	std::vector<OtzCrcChunk> chunks;
-	std::vector<uint32_t> infl, zst, d64;
+	std::vector<uint32_t> infl, zst, d64, xz;
 	uint64_t need = 0;
 	for (int pass = 0; pass < 2; pass++) {
 		for (uint32_t i = 0; i < n; i++) {
@@ -528,6 +544,8 @@ extern "C" int otz_plan_create(otz_ctx *c, const otz_entry *ents, uint32_t n, co
 			zst.push_back(i);
 		} else if (ents[i].method == OTZ_M_DEFLATE64 && !(ents[i].flags & OTZ_EF_CHUNK)) {
 			d64.push_back(i);   // never on the two-phase path: its 32-bit records hold neither 64 KiB distances nor long lengths
+		} else if (ents[i].method == OTZ_M_XZ && !(ents[i].flags & OTZ_EF_CHUNK)) {
+			xz.push_back(i);
 		}
 		if (!(opts->verify_only && ents[i].method == OTZ_M_STORE)) {
 			need = std::max<uint64_t>(need, ents[i].out_ofs + ents[i].uncomp_size);
@@ -569,6 +587,17 @@ extern "C" int otz_plan_create(otz_ctx *c, const otz_entry *ents, uint32_t n, co
 		p->n_d64_big += ents[i].uncomp_size >= big_bytes;
 	}
 	p->n_d64 = (uint32_t)d64.size();
+	// XZ: longest first; every entry gets the segment slots its declared size can need
+	std::stable_sort(xz.begin(), xz.end(), [&](uint32_t a, uint32_t b) { return ents[a].comp_size > ents[b].comp_size; });
+	std::vector<XzEnt> xe(xz.size());
+	uint64_t xz_slots = 0;
+	for (size_t k = 0; k < xz.size(); k++) {
+		xe[k].first = (uint32_t)xz_slots;
+		xe[k].cap = ents[xz[k]].uncomp_size / XZ_SEG_MIN + 1u;
+		xz_slots += xe[k].cap;
+	}
+	p->n_xz = (uint32_t)xz.size();
+	p->n_xz_slots = (uint32_t)xz_slots;
 	p->n_chunks = (uint32_t)chunks.size();
 	p->n_inflate = (uint32_t)infl.size();
 	p->n_zstd = (uint32_t)zst.size();
@@ -613,7 +642,8 @@ extern "C" int otz_plan_create(otz_ctx *c, const otz_entry *ents, uint32_t n, co
 	}
 	if ((rc = upload(&p->d_ents, ev, c->stream)) || (rc = upload(&p->d_chunks, chunks, c->stream)) ||
 		(rc = upload(&p->d_inflate_list, infl, c->stream)) || (rc = upload(&p->d_zstd_list, zst, c->stream)) ||
-		(rc = upload(&p->d_zchunks, zchunks, c->stream)) || (rc = upload(&p->d_d64_list, d64, c->stream))) {
+		(rc = upload(&p->d_zchunks, zchunks, c->stream)) || (rc = upload(&p->d_d64_list, d64, c->stream)) ||
+		(rc = upload(&p->d_xz_list, xz, c->stream)) || (rc = upload(&p->d_xz_ent, xe, c->stream))) {
 		otz_plan_destroy(c, p);
 		return rc;
 	}
@@ -621,6 +651,7 @@ extern "C" int otz_plan_create(otz_ctx *c, const otz_entry *ents, uint32_t n, co
 	if (cudaMalloc(&p->d_est, n1 * sizeof(OtzEntryState)) != cudaSuccess || cudaMalloc(&p->d_status, n1 * 4) != cudaSuccess ||
 		cudaMalloc(&p->d_acc, n1 * 4) != cudaSuccess || cudaMalloc(&p->d_crc, n1 * 4) != cudaSuccess ||
 		cudaMalloc(&p->d_produced, n1 * 4) != cudaSuccess ||
+		cudaMalloc(&p->d_xz_segs, std::max<uint64_t>(xz_slots, 1) * sizeof(XzSeg)) != cudaSuccess ||
 		cudaMalloc(&p->d_counter, 256) != cudaSuccess) {
 		otz_plan_destroy(c, p);
 		return fail_cuda(cudaGetLastError(), "cudaMalloc(plan)");
@@ -1069,6 +1100,44 @@ static int dispatch_deflate64(otz_ctx *c, otz_plan *p, const uint8_t *d_archive,
 	return rc;
 }
 
+template <int LCLP>
+static int launch_lzma(otz_ctx *c, otz_plan *p, const uint8_t *d_archive, uint8_t *d_out, uint32_t *d_work, const uint32_t *d_n_class) {
+	const size_t smem = sizeof(XzSmem<LCLP>);
+	int per_sm = 0;
+	CK(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_lzma<LCLP>, 32, smem));
+	const uint32_t grid = std::max(1u, std::min((uint32_t)(c->sm_count * std::max(per_sm, 1)), p->n_xz_slots));
+	k_lzma<LCLP><<<grid, 32, smem, c->stream_xz>>>(d_archive, d_out, p->d_ents, p->d_est, p->d_xz_list, p->d_xz_ent, p->d_xz_segs,
+		p->n_xz_slots, d_work, d_n_class);
+	c->launches++;
+	CK(cudaGetLastError());
+	return OTZ_SUCCESS;
+}
+
+// XZ entries (k_xz.cuh): walk, decode (one launch per shared-memory class) and verdicts on a stream of their own, forked
+// behind k_resolve and joined before the CRC.  Words of d_counter: 26 / 27 = slot counters of the two k_lzma launches,
+// 28 / 29 = segments of each class (counted by the walk; a launch whose class has none returns at once).
+static int dispatch_xz(otz_ctx *c, otz_plan *p, const uint8_t *d_archive, uint8_t *d_out) {
+	cudaStream_t st = c->stream_xz;
+	CK(cudaEventRecord(c->ev_xz_fork, c->stream));
+	CK(cudaStreamWaitEvent(st, c->ev_xz_fork, 0));
+	const uint32_t *t0 = reinterpret_cast<const uint32_t *>(reinterpret_cast<const uint8_t *>(c->d_tabs) + offsetof(OtzCrcTables, t0));
+	k_xz_walk<<<(p->n_xz + 127) / 128, 128, 0, st>>>(d_archive, p->d_ents, p->d_est, p->d_status, p->d_xz_list, p->n_xz, p->d_xz_ent,
+		p->d_xz_segs, t0, p->d_counter + 28);
+	c->launches++;
+	int rc = launch_lzma<3>(c, p, d_archive, d_out, p->d_counter + 26, p->d_counter + 28);
+	if (rc == OTZ_SUCCESS) {
+		rc = launch_lzma<4>(c, p, d_archive, d_out, p->d_counter + 27, p->d_counter + 29);
+	}
+	if (rc) {
+		return rc;
+	}
+	k_xz_finish<<<(p->n_xz + 7) / 8, 256, 0, st>>>(d_out, p->d_ents, p->d_status, p->d_produced, p->d_xz_list, p->n_xz, p->d_xz_ent,
+		p->d_xz_segs);
+	c->launches++;
+	CK(cudaEventRecord(c->ev_xz_join, st));
+	return OTZ_SUCCESS;
+}
+
 extern "C" int otz_extract_run(otz_ctx *c, otz_plan *p, const uint8_t *d_archive, uint64_t archive_len, uint8_t *d_out,
 	uint64_t out_len) {
 	if (!c || !p || (!d_archive && archive_len)) {
@@ -1098,6 +1167,12 @@ extern "C" int otz_extract_run(otz_ctx *c, otz_plan *p, const uint8_t *d_archive
 	int d64_joins = 0;
 	if (p->n_d64) {
 		const int rc = dispatch_deflate64(c, p, d_archive, d_out, &d64_joins);
+		if (rc) {
+			return rc;
+		}
+	}
+	if (p->n_xz) {
+		const int rc = dispatch_xz(c, p, d_archive, d_out);
 		if (rc) {
 			return rc;
 		}
@@ -1198,6 +1273,9 @@ extern "C" int otz_extract_run(otz_ctx *c, otz_plan *p, const uint8_t *d_archive
 	}
 	for (int k = 0; k < d64_joins; k++) {
 		CK(cudaStreamWaitEvent(s, c->ev_d64_join[k], 0));
+	}
+	if (p->n_xz) {
+		CK(cudaStreamWaitEvent(s, c->ev_xz_join, 0));
 	}
 	if (c->profile) {
 		CK(cudaEventRecord(pev[2], s));

@@ -8,7 +8,7 @@ import ctypes as C
 from .native import Lib
 
 ZIP_RDONLY, ZIP_CREATE, ZIP_EXCL, ZIP_TRUNCATE = 0, 1, 2, 8
-ZIP_CM_STORE, ZIP_CM_DEFLATE, ZIP_CM_DEFLATE64 = 0, 8, 9
+ZIP_CM_STORE, ZIP_CM_DEFLATE, ZIP_CM_DEFLATE64, ZIP_CM_XZ = 0, 8, 9, 95
 ZIP_EM_NONE, ZIP_EM_TRAD_PKWARE, ZIP_EM_AES_128, ZIP_EM_AES_192, ZIP_EM_AES_256 = 0, 1, 0x0101, 0x0102, 0x0103
 
 
